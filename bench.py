@@ -28,6 +28,12 @@ One JSON line is printed by rank 0:
                    one: device-resident value, step-kernel time, roofline fraction, end-to-end value (N=1 only)
 ``--impl reference`` times the reference's own CPU implementation of the path on all host cores, on the same config and
 step counts, and prints the same line shape (rank 0 only under torchrun).
+
+``--dump-outputs DIR`` writes what the last timed step of the device-resident path left in the engine's per-environment
+buffers (state, actions, rewards, dones, observations, masks) as ``DIR/<name>.npy``, at most 64 MB in all whatever N
+(a fixed seeded sample of the environments of every rank, ``DIR/env_index.npy``), so that two builds can be compared
+output for output: the inputs are seeded, so they are the same on every run.  ``--steps`` is the number of timed steps
+of every GPU leg and of ``--impl reference``; only ``cpu_baseline`` times a bounded sample of its own.
 """
 from __future__ import annotations
 
@@ -60,6 +66,7 @@ WORKLOADS = {
 KERNELS = {'wildfire': 'wildfire_step_kernel', 'rideshare': 'rideshare_tile_kernel / rideshare_step_kernel (by batch size)',
            'cybersecurity': 'cyber_step_tiled_kernel'}
 SEED, SAMPLER = 2026, 2026
+DUMP_ENVS, DUMP_BYTES = 4096, 64 << 20  # --dump-outputs: at most this many sampled environments, this many bytes
 
 
 def algorithmic_bytes(domain: str, raw, present: float = 0.0) -> float:
@@ -311,7 +318,7 @@ def run_reference(args):
         source = ('UNMODIFIED reference (oracle/_ref/free_range_zoo, imported under oracle/ref_shim.py), '
                   f'{args.workload}_v0.parallel_env(device="cpu", single_seeding=True, buffer_size=0)')
     else:  # the copy of the reference did not travel: fall back to the numpy restatement and say so
-        envs_per_process, K = min(envs_per_process, cpu_sample_size(args.workload)[0]), min(K, 10)
+        envs_per_process = min(envs_per_process, cpu_sample_size(args.workload)[0])
         value, executed = cpu_throughput('port', args.workload, cores, envs_per_process, K)
         source = f'numpy oracle port (oracle/{spec["domain"]}.py): oracle/_ref is absent'
     wall = time.perf_counter() - start
@@ -556,11 +563,44 @@ def summarize_workload(name: str, B: int, device, K: int, W: int, e2e: str):
         record['e2e'] = {'value': B / (ms * 1e-3), 'ms_per_step': ms, 'h2d_bytes_per_step': h2d, 'd2h_bytes_per_step': d2h,
                          'slices': slices, 'timing': 'CUDA events around K step_host calls'}
     else:
-        ms = h.host_wall_clock(5, 2)
-        record['e2e'] = {'value': B / (ms * 1e-3), 'ms_per_step': ms, 'timing': 'host clock per step_host call, 5 steps'}
+        ms = h.host_wall_clock(K, W)
+        record['e2e'] = {'value': B / (ms * 1e-3), 'ms_per_step': ms, 'timing': f'host clock per step_host call, {K} steps'}
     del h
     torch.cuda.empty_cache()
     return record
+
+
+def dump_outputs(raw, B: int, directory: str, rank: int = 0, world: int = 1, dist=None):
+    """Every per-environment buffer the step kernels write as ``<name>.npy``: float32, or float64 for 32- and 64-bit
+    integers and doubles so that every value is exact.  The configuration tables bound next to them, the initial-state
+    copies, the control block and injected uniforms are left out.  Rows are environments: all ``world * B`` of them, or a
+    fixed seeded sample when that would exceed DUMP_ENVS environments or DUMP_BYTES in all; ``env_index.npy`` lists their
+    global indices.  Rank r steps environments [r * B, (r + 1) * B); rank 0 gathers the rows and writes the files."""
+    import numpy as np
+    import torch
+    skipped = {'control', 'cell_reward', 'cell_ignition', 'range_mask', 'cell_agents', 'schedule', 'schedule_index',
+               'score_lut'}
+    arrays = {name: tensor for name, tensor in raw._bound.items() if tensor is not None and name not in skipped
+              and not name.startswith('init_') and not name.endswith('_uniforms')}
+    wide = {name: tensor.element_size() >= 4 and (not tensor.is_floating_point() or tensor.dtype == torch.float64)
+            for name, tensor in arrays.items()}
+    env_bytes = 8 + sum(tensor[0].numel() * (8 if wide[name] else 4) for name, tensor in arrays.items())
+    total = world * B
+    count = min(total, DUMP_ENVS, DUMP_BYTES // env_bytes)
+    index = np.arange(total) if count == total else np.sort(np.random.default_rng(SEED).choice(total, count, replace=False))
+    mine = index[(index >= rank * B) & (index < (rank + 1) * B)] - rank * B
+    rows = torch.from_numpy(mine).to(raw.device)
+    values = {name: tensor.index_select(0, rows).cpu().numpy() for name, tensor in arrays.items()}
+    if world > 1:
+        shards = [None] * world if rank == 0 else None
+        dist.gather_object(values, shards, dst=0)
+        if rank != 0:
+            return
+        values = {name: np.concatenate([shard[name] for shard in shards]) for name in arrays}
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, 'env_index.npy'), index.astype(np.float64))
+    for name, array in values.items():
+        np.save(os.path.join(directory, f'{name}.npy'), array.astype(np.float64 if wide[name] else np.float32))
 
 
 def run_engine(args):
@@ -593,6 +633,8 @@ def run_engine(args):
     per_replay, windows = h.graph_windows(max(1, args.windows))
     graph_ms = sorted(windows)[len(windows) // 2]
     value = world * B * K / (graph_ms * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(raw, B, args.dump_outputs, rank, world, dist)
 
     eager_ms, kernel_ms, mean_tasks = h.kernel_times()
     bytes_per_env = algorithmic_bytes(domain, raw, mean_tasks)
@@ -699,7 +741,13 @@ def main():
                         help='slices of the pipelined host-buffer step of the e2e leg (0 = the engine\'s default)')
     parser.add_argument('--skip-other-workloads', action='store_true',
                         help='only the named workload (skips config.other_workloads)')
+    parser.add_argument('--dump-outputs', metavar='DIR',
+                        help='write the outputs of the last timed step as DIR/<name>.npy (engine only)')
     args = parser.parse_args()
+    if args.steps < 1:
+        parser.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'engine':
+        parser.error('--dump-outputs writes the engine\'s outputs; --impl reference has none to write')
     if args.impl == 'reference':
         run_reference(args)
     else:
