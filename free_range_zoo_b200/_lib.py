@@ -145,6 +145,23 @@ class GatherArray(C.Structure):
                 ('groups', C.c_int32), ('reserved', C.c_int32)]
 
 
+class ObsArray(C.Structure):
+    """FrzObsArray (include/frz_obs.h): one array of the compact observation download."""
+    _fields_ = [('src', C.c_void_p), ('dst', C.c_void_p), ('host', C.c_void_p), ('kind', C.c_int32), ('src_type', C.c_int32),
+                ('dst_type', C.c_int32), ('groups', C.c_int32), ('capacity', C.c_int32), ('src_columns', C.c_int32),
+                ('column_first', C.c_int32), ('columns', C.c_int32)]
+
+
+class ObsDownload(C.Structure):
+    """FrzObsDownload (include/frz_obs.h): counts, host offsets, device scratch and the arrays of one download."""
+    _fields_ = [('counts', C.c_void_p), ('offsets', C.c_void_p), ('host_offsets', C.c_void_p), ('scan', C.c_void_p),
+                ('scratch', C.c_void_p),
+                ('status', C.c_void_p), ('arrays', C.POINTER(ObsArray)), ('array_count', C.c_int32),
+                ('mask_groups', C.c_int32)]
+
+
+OBS_DENSE, OBS_ROWS, OBS_MASK_BITS = 0, 1, 2
+OBS_I32, OBS_I16, OBS_I8, OBS_U8, OBS_F32 = 0, 1, 2, 3, 4
 HOST_ACTIONS_I32, HOST_ACTIONS_I16, HOST_ACTIONS_I8 = 0, 1, 2
 ABI_VERSION = 4
 
@@ -189,6 +206,7 @@ def library() -> C.CDLL:
     lib.frz_wildfire_tile_random_layout.argtypes = [C.POINTER(WildfireParams), C.POINTER(C.c_uint32), C.POINTER(C.c_int8)]
     lib.frz_gather_live_rows.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(GatherArray), C.c_int32,
                                          C.c_void_p]
+    lib.frz_observe_compact.argtypes = [C.POINTER(ObsDownload), C.c_int32, C.c_void_p]
     if lib.frz_version() != ABI_VERSION:
         raise RuntimeError(f'libfrz.so ABI version {lib.frz_version()} != {ABI_VERSION}; rebuild the library')
     lib.frz_control_restore.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p]
@@ -225,9 +243,9 @@ def pointer(tensor: torch.Tensor | None) -> int | None:
     return None if tensor is None else tensor.data_ptr()
 
 
-def exported_symbols():
-    """Every extern "C" symbol include/frz.h declares (used by the CPU-side ABI test)."""
+def exported_symbols(header: str = 'frz.h'):
+    """Every extern "C" symbol an include/ header declares (used by the CPU-side ABI tests)."""
     import re
-    header = os.path.join(os.path.dirname(_HERE), 'include', 'frz.h')
+    header = os.path.join(os.path.dirname(_HERE), 'include', header)
     text = open(header).read()
     return sorted(set(re.findall(r'\b(frz_[a-z_]+)\s*\(', text)))

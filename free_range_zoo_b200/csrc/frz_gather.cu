@@ -9,43 +9,10 @@
 // (environment, row block) segment copies its rows to the packed position.  All of it is plain HBM streaming.
 #include <algorithm>
 
-#include "frz_common.cuh"
+#include "frz_scan.cuh"
 
 namespace frz {
 namespace {
-
-constexpr int kScanThreads = 256;
-constexpr int kScanItems = 4;  // counts per thread
-constexpr int kScanBlock = kScanThreads * kScanItems;
-
-__device__ __forceinline__ int warp_inclusive_scan(int value, int lane) {
-#pragma unroll
-  for (int d = 1; d < 32; d <<= 1) {
-    const int below = __shfl_up_sync(kFullMask, value, d);
-    if (lane >= d) value += below;
-  }
-  return value;
-}
-
-// exclusive scan of one int per thread over the CTA; returns this thread's prefix, *total = the CTA's sum
-__device__ __forceinline__ int cta_exclusive_scan(int value, int* total) {
-  __shared__ int warp_sums[32];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int inclusive = warp_inclusive_scan(value, lane);
-  if (lane == 31) warp_sums[warp] = inclusive;
-  __syncthreads();
-  if (warp == 0) {
-    const int warps = (blockDim.x + 31) >> 5;
-    const int sum = lane < warps ? warp_sums[lane] : 0;
-    const int scanned = warp_inclusive_scan(sum, lane);
-    warp_sums[lane] = scanned - sum;  // exclusive prefix of the warps
-    if (lane == 31) *total = scanned;
-  }
-  __syncthreads();
-  const int result = inclusive - value + warp_sums[warp];
-  __syncthreads();  // (warp_sums is reused by the next call)
-  return result;
-}
 
 // block_sums[i] = sum of counts[i * kScanBlock ... )
 __global__ void __launch_bounds__(kScanThreads) gather_block_sums(const int32_t* __restrict__ counts, int B,

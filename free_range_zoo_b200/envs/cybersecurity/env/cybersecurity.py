@@ -18,6 +18,7 @@ from free_range_zoo_b200 import _lib
 from free_range_zoo_b200.envs.cybersecurity.env.structures.state import CybersecurityState
 from free_range_zoo_b200.utils.containers import LazyDict, ObservationDict, jagged_indices_from_mask
 from free_range_zoo_b200.utils.conversions import batched_aec_to_batched_parallel
+from free_range_zoo_b200.utils import compact
 from free_range_zoo_b200.utils.env import BatchedAECEnv
 from free_range_zoo_b200.utils.spaces import BatchedActionSpace, Space
 
@@ -95,6 +96,14 @@ def flatten_configuration(config, max_steps, show_bad_actions: bool, env_offset:
         lut = danger_score_table(threat, mitigation, float(nc.temperature))
         p.lut_bits = n_att + n_def
     return p, lut
+
+
+def compact_bounds(params) -> Dict[str, int]:
+    """Largest |value| of the integer observations, from the configuration (utils/compact.py picks the types): task
+    rows hold (state, criticality), task counts at most every subnetwork."""
+    N = int(params.num_nodes)
+    criticality = max(abs(int(params.criticality[n])) for n in range(N))
+    return dict(task_obs=max(int(params.num_states) - 1, criticality), agent_task_count=N)
 
 
 class raw_env(BatchedAECEnv):
@@ -247,6 +256,18 @@ class raw_env(BatchedAECEnv):
         dense = dict(attacker_self=self._attacker_self, defender_self=self._defender_self, task_obs=self._task_obs,
                      monitored=self._monitored, agent_task_count=self._agent_task_count)
         return dense, {}
+
+    def _compact_schema(self):
+        """Compact download (utils/compact.py): task rows and counts narrowed; the float arrays and ``monitored`` as
+        they are.  Every environment has all subnetworks as tasks, so everything is dense."""
+        bounds = compact_bounds(self._params)
+        return compact.Schema(capacity=int(self._params.num_nodes), arrays=[
+            compact.dense('attacker_self', self._attacker_self),
+            compact.dense('defender_self', self._defender_self),
+            compact.dense('task_obs', self._task_obs, bound=bounds['task_obs']),
+            compact.dense('monitored', self._monitored),
+            compact.dense('agent_task_count', self._agent_task_count, bound=bounds['agent_task_count']),
+        ])
 
     def update_actions(self) -> None:
         """Recompute task counts from the current state (cybersecurity.py:414-457); only needed after manual edits."""

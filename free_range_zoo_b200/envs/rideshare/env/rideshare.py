@@ -18,6 +18,7 @@ from free_range_zoo_b200.envs.rideshare.env.structures.state import RideshareSta
 from free_range_zoo_b200.utils.containers import (LazyDict, ObservationDict, jagged_indices_from_mask,
                                                   jagged_rows_from_mask)
 from free_range_zoo_b200.utils.conversions import batched_aec_to_batched_parallel
+from free_range_zoo_b200.utils import compact
 from free_range_zoo_b200.utils.env import BatchedAECEnv
 from free_range_zoo_b200.utils.spaces import BatchedActionSpace, Space
 
@@ -71,6 +72,19 @@ def flatten_configuration(config, max_steps, parallel_envs: int, env_offset: int
                  'long_wait_cost'):
         setattr(p, name, float(getattr(rc, name)))
     return p, schedule
+
+
+def compact_bounds(config, params, max_steps) -> Dict[str, int]:
+    """Largest |value| of the integer observations, from the configuration (utils/compact.py picks the types): task
+    rows (y, x, dest_y, dest_x, accepted_by, riding_by, fare, entered) hold grid positions, driver indices or the
+    padding value, the schedule's fares and entry steps (at most the horizon); self observations (y, x, #accepted,
+    #riding) grid positions and passenger counts."""
+    H, W, A, K = int(config.grid_height), int(config.grid_width), int(params.num_agents), int(params.capacity)
+    schedule = torch.as_tensor(config.passenger_config.schedule).reshape(-1, 7)
+    max_fare = int(schedule[:, 6].abs().max()) if schedule.numel() else 0
+    horizon = 2**31 - 1 if max_steps is None else max(int(max_steps), int(params.schedule_horizon))
+    return dict(task_obs=max(H - 1, W - 1, A - 1, -_lib.PAD, max_fare, horizon), self_obs=max(H - 1, W - 1, K),
+                agent_task_count=K)
 
 
 def schedule_index(schedule: np.ndarray, horizon: int) -> np.ndarray:
@@ -199,6 +213,17 @@ class raw_env(BatchedAECEnv):
         dense = dict(self_obs=self._self_obs, agent_task_count=self._agent_task_count)
         ragged = dict(task_obs=(self._task_obs, 1), task_mask=(self._task_mask, len(self.possible_agents)))
         return dense, ragged
+
+    def _compact_schema(self):
+        """Compact download (utils/compact.py): live task rows, the task mask as bits, self observations and counts."""
+        A = len(self.possible_agents)
+        bounds = compact_bounds(self.config, self._params, self.max_steps)
+        return compact.Schema(capacity=self._capacity, mask_groups=A, arrays=[
+            compact.rows('task_obs', self._task_obs, bound=bounds['task_obs']),
+            compact.mask('task_mask', self._task_mask, groups=A),
+            compact.dense('self_obs', self._self_obs, bound=bounds['self_obs']),
+            compact.dense('agent_task_count', self._agent_task_count, bound=bounds['agent_task_count']),
+        ])
 
     def update_actions(self) -> None:
         """Recompute task lists from the current table (rideshare.py:368-395); only needed after manual edits."""

@@ -18,6 +18,7 @@ from free_range_zoo_b200.envs.wildfire.env.structures.state import WildfireState
 from free_range_zoo_b200.utils.containers import (LazyDict, ObservationDict, jagged_from_padded,
                                                   jagged_indices_from_mask)
 from free_range_zoo_b200.utils.conversions import batched_aec_to_batched_parallel
+from free_range_zoo_b200.utils import compact
 from free_range_zoo_b200.utils.env import BatchedAECEnv
 from free_range_zoo_b200.utils.spaces import BatchedActionSpace, Space
 
@@ -129,6 +130,14 @@ def flatten_configuration(config, max_steps, show_bad_actions: bool, env_offset:
             for c in np.nonzero(chebyshev <= reach)[0]:
                 range_mask[a, e, c >> 5] |= np.uint32(1 << (c & 31))
     return p, _np(rc.fire_rewards, np.float32).reshape(-1), _np(fc.ignition_temp, np.int32).reshape(-1), range_mask
+
+
+def compact_bounds(config) -> Dict[str, int]:
+    """Largest |value| of the integer observations, from the configuration (utils/compact.py picks the types)."""
+    H, W, fc = int(config.grid_height), int(config.grid_width), config.fire_config
+    max_fire_type = max(int(fc.max_fire_type), int(torch.as_tensor(fc.fire_types).abs().max()))
+    return dict(task_obs=max(H - 1, W - 1, max_fire_type, int(fc.num_fire_states) - 1),  # (y, x, fire type, intensity)
+                agent_task_count=H * W)
 
 
 def transpose_range_mask(range_mask: np.ndarray, cells: int) -> np.ndarray:
@@ -295,6 +304,20 @@ class raw_env(BatchedAECEnv):
         dense = dict(self_obs=self._self_obs, agent_task_count=self._agent_task_count)
         ragged = dict(task_obs=(self._task_obs, 1), action_mask=(self._action_mask, len(self.possible_agents)))
         return dense, ragged
+
+    def _compact_schema(self):
+        """Compact download (utils/compact.py): live task rows and the action mask as bits; of ``self_obs`` only the
+        suppressant -- y, x and power are the configuration's and are restored by ``unpack()``."""
+        A, p = len(self.possible_agents), self._params
+        bounds = compact_bounds(self.config)
+        fill = torch.tensor([[float(p.agent_y[a]), float(p.agent_x[a]), p.agent_power[a], 0.0] for a in range(A)],
+                            dtype=torch.float32)
+        return compact.Schema(capacity=self.max_y * self.max_x, mask_groups=A, arrays=[
+            compact.rows('task_obs', self._task_obs, bound=bounds['task_obs']),
+            compact.mask('action_mask', self._action_mask, groups=A),
+            compact.dense('self_obs', self._self_obs, columns=(3, 1), fill=fill),
+            compact.dense('agent_task_count', self._agent_task_count, bound=bounds['agent_task_count']),
+        ])
 
     def update_actions(self) -> None:
         """Recompute task counts / masks from the current state (wildfire.py:587-666). The fused step already does

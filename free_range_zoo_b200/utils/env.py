@@ -27,6 +27,7 @@ from typing import Any, Dict, List, Optional, Tuple
 import torch
 
 from free_range_zoo_b200 import _lib
+from free_range_zoo_b200.utils import compact
 from free_range_zoo_b200.utils.configuration import Configuration
 from free_range_zoo_b200.utils.containers import ObservationDict
 from free_range_zoo_b200.utils.selector import AgentSelector
@@ -434,8 +435,27 @@ class BatchedAECEnv(ABC):
         out['bytes'] = moved
         return out
 
+    def _compact_schema(self) -> compact.Schema:
+        """The domain's compact observation format (utils/compact.py): which array is narrowed to which type, from
+        bounds the configuration guarantees.  Domain hook."""
+        raise NotImplementedError
+
+    def _compact_download(self) -> compact.CompactDownload:
+        download = getattr(self, '_compact', None)
+        if download is None or download.key != self.max_steps:  # (rideshare bounds depend on the horizon)
+            download = compact.CompactDownload(self._compact_schema(), self.environment_task_count, key=self.max_steps)
+            self._compact = download
+        return download
+
+    def _enqueue_compact(self) -> compact.CompactDownload:
+        """The compact download of the current state (frz_observe_compact), on the current stream of the device."""
+        download = self._compact_download()
+        _lib.check(self._lib.frz_observe_compact(ctypes.byref(download.block), self.parallel_envs, self._stream()),
+                   'frz_observe_compact')
+        return download
+
     @torch.no_grad()
-    def gather_observations(self) -> Dict[str, Any]:
+    def gather_observations(self, compact: bool = False) -> Dict[str, Any]:
         """The observations of the current state in page-locked HOST memory, packed like the reference's jagged nested
         tensors (a value buffer + offsets; wildfire.py:669-717, rideshare.py:398-467): ``counts`` int32 [B] live tasks
         per environment, ``offsets`` int32 [B + 1] their exclusive prefix sum, the dense arrays (``self_obs``,
@@ -443,15 +463,23 @@ class BatchedAECEnv(ABC):
         g of array ``name`` is ``out[name][offsets[b] * groups + g * counts[b] :][:counts[b]]`` (groups = 1 for task
         observations, = agents for the action / task masks).  The live rows are compacted on the device
         (``frz_gather_live_rows``) so that each array crosses PCIe in one copy of exactly its live bytes.  The
-        returned tensors are overwritten by the next call.  ``out['bytes']`` = bytes copied device -> host."""
+        returned tensors are overwritten by the next call.  ``out['bytes']`` = bytes copied device -> host.
+
+        ``compact=True`` returns the same observations in the compact format instead (a ``CompactObservations``,
+        utils/compact.py: narrow integers, bit masks, no configuration constants; ``.unpack()`` gives this dict), encoded
+        on the device and stored straight into page-locked host buffers: one synchronisation, fewer bytes."""
         with torch.cuda.device(self.device):
+            if compact:
+                download = self._enqueue_compact()
+                torch.cuda.current_stream(self.device).synchronize()
+                return download.result()
             state = self._gather_state()
             self._enqueue_gather(state)
             torch.cuda.current_stream(self.device).synchronize()
             return self._finish_gather(state)
 
     @torch.no_grad()
-    def step_host(self, host_actions: torch.Tensor, chunks: Optional[int] = None, observations: bool = False
+    def step_host(self, host_actions: torch.Tensor, chunks: Optional[int] = None, observations: bool | str = False
                   ) -> Tuple[torch.Tensor, ...]:
         """One environment step for callers that live on the host: ``host_actions`` is a page-locked int32 -- or int16 /
         int8 (at most 127 tasks per environment), which halve / quarter the upload and are widened on the device --
@@ -463,7 +491,11 @@ class BatchedAECEnv(ABC):
         (``frz_<domain>_step_host``, include/frz.h); the results are bit-identical.  Observations, masks and counts stay
         on the device as usual -- unless ``observations=True``: then the call also returns, as a fourth element, what
         ``gather_observations()`` returns (the next observations in host memory, packed), which is what a policy that
-        runs on the CPU needs for its next decision."""
+        runs on the CPU needs for its next decision.  ``observations='compact'`` returns them as
+        ``gather_observations(compact=True)`` does: encoded on the device after the step and stored into page-locked
+        host buffers, with one stream synchronisation for the whole call."""
+        if not (isinstance(observations, bool) or (isinstance(observations, str) and observations == 'compact')):
+            raise ValueError(f"observations must be False, True or 'compact', not {observations!r}")
         B, A = self.parallel_envs, len(self.possible_agents)
         if (host_actions.device.type != 'cpu' or host_actions.dtype not in (torch.int32, torch.int16, torch.int8)
                 or not host_actions.is_contiguous() or tuple(host_actions.shape) != (B, A, 2)
@@ -487,6 +519,11 @@ class BatchedAECEnv(ABC):
         if not observations:
             main.synchronize()
             return state['rewards'], state['terminated'], state['truncated']
+        if observations == 'compact':
+            with torch.cuda.stream(main):
+                download = self._enqueue_compact()
+            main.synchronize()
+            return state['rewards'], state['terminated'], state['truncated'], download.result()
         with torch.cuda.stream(main):  # compaction + fixed-size downloads ride on the same synchronisation
             gather = self._gather_state()
             self._enqueue_gather(gather)
