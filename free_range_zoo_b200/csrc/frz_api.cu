@@ -36,13 +36,15 @@ __global__ void control_init_kernel(FrzControl* control, uint64_t seed) {
   control->agents_with_tasks = 0;
 }
 
-// a checkpoint's random stream: every draw is Philox(seed; env, step, event), so (seed, step) is the whole state
+// a checkpoint's random stream: every draw is Philox(seed; env, step, event), so (seed, step) is the whole state.  The
+// published flags are left to the refresh that follows (they depend on the restored state arrays); faults recorded
+// before the restore belong to the abandoned run.
 __global__ void control_restore_kernel(FrzControl* control, uint64_t seed, uint64_t step) {
   control->seed = seed;
   control->step = step;
   control->ctas_done = 0;
   control->alive_acc = 0;
-  control->alive = 3u;
+  control->error_word = 0;
   control->agents_with_tasks_acc = 0;
 }
 

@@ -247,8 +247,10 @@ __device__ __forceinline__ void fence_async_shared() { asm volatile("fence.proxy
 // Called by every CTA once, after its last environment.
 //   alive_bits: bit0 = this CTA saw an env that is still not terminated, bit1 = one that is still not truncated
 //   agent_bits: bit a = agent a has at least one task in some env of this CTA (after this launch)
-// The last CTA to arrive publishes the accumulated flags for the next launch and advances the step counter -- every
-// CTA read control->step / alive / agents_with_tasks at its start, so no reader is left when they change.
+// The last CTA to arrive publishes the accumulated flags for the next launch (a step and a refresh both do: a refresh
+// follows every reset, checkpoint restore and hand edit of the state, whose done flags the next step must see) and, after
+// a step, advances the step counter -- every CTA read control->step / alive / agents_with_tasks at its start, so no
+// reader is left when they change.
 enum Publish { kPublishNothing = 0, kPublishRefresh = 1, kPublishStep = 2 };
 
 __device__ __forceinline__ void finish_launch(FrzControl* control, unsigned alive_bits, unsigned fault_bits,
@@ -279,6 +281,7 @@ __device__ __forceinline__ void finish_launch(FrzControl* control, unsigned aliv
         control->step += 1;
       }
       if (publish != kPublishNothing) control->agents_with_tasks = agents;
+      if (publish == kPublishRefresh) control->alive = alive;
       control->ctas_done = 0u;
     }
   }

@@ -288,6 +288,8 @@ cyber_step_kernel(const __grid_constant__ FrzCyberParams p, const __grid_constan
       r.network_uniforms = io.network_uniforms != nullptr ? io.network_uniforms + e * N : nullptr;
       r.agent_uniforms = io.agent_uniforms != nullptr ? io.agent_uniforms + e * n_agents : nullptr;
       cyber_env_step<MODE, 0, 0, 0>(p, r, io.score_lut, philox, step, p.env_offset + env, alive_bits, faults);
+      // refresh: the done flags as a reset, a restore or a hand edit left them
+      if (MODE == kCyRefresh) alive_bits |= (io.terminated[e] ? 0u : 1u) | (io.truncated[e] ? 0u : 2u);
     }
   }
   finish_launch(control, alive_bits, faults, 0u,
@@ -545,7 +547,6 @@ __global__ void cyber_restore_kernel(const FrzCyberParams p, const FrzCyberBuffe
     io.truncated[env] = 0;
     io.num_moves[env] = 0;
   }
-  if (blockIdx.x == 0 && threadIdx.x == 0) io.control->alive = 3u;
 }
 
 // Uniform over the legal choices of spaces/actions.py:11-99:

@@ -461,6 +461,8 @@ rideshare_step_kernel(const __grid_constant__ FrzRideshareParams p, const __grid
           io.truncated[env] = truncated;
         }
         if (valid) alive_bits |= 1u | (truncated ? 0u : 2u);  // rideshare never terminates (rideshare.py:252)
+      } else if (valid) {  // refresh: the done flags as a reset, a restore or a hand edit left them
+        alive_bits |= (io.terminated[env] ? 0u : 1u) | (io.truncated[env] ? 0u : 2u);
       }
 
       // ------------------------------------------------------------------ publish
@@ -1059,6 +1061,8 @@ rideshare_tile_kernel(const __grid_constant__ FrzRideshareParams p, const __grid
             io.num_moves[env] = moves;
             io.truncated[env] = truncated;
             alive_bits |= 1u | (truncated ? 0u : 2u);  // rideshare never terminates (rideshare.py:252)
+          } else {  // refresh: the done flags as a reset, a restore or a hand edit left them
+            alive_bits |= (io.terminated[env] ? 0u : 1u) | (io.truncated[env] ? 0u : 2u);
           }
           io.env_task_count[env] = n_rows;
         }
@@ -1098,7 +1102,6 @@ __global__ void rideshare_restore_kernel(const FrzRideshareParams p, const FrzRi
       io.num_moves[env] = 0;
     }
   }
-  if (blockIdx.x == 0 && threadIdx.x == 0) io.control->alive = 3u;
 }
 
 // Uniform over [task 0 .. task n-1, noop]; the action id of a task is the passenger's state (0 accept / 1 pick /

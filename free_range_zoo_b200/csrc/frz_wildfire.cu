@@ -817,6 +817,8 @@ wildfire_step_kernel(const __grid_constant__ FrzWildfireParams p, const __grid_c
         truncated = moves >= p.max_steps;
         cumulative = __fadd_rn(cumulative, reward);
         if (valid) alive_bits |= (terminated ? 0u : 1u) | (truncated ? 0u : 2u);
+      } else if (valid) {  // refresh: the done flags as a reset, a restore or a hand edit left them
+        alive_bits |= (io.terminated[e] ? 0u : 1u) | (io.truncated[e] ? 0u : 2u);
       }
 
       // ------------------------------------------------------------------ update_actions / update_observations
@@ -1015,7 +1017,6 @@ __global__ void wildfire_restore_kernel(const FrzWildfireParams p, const FrzWild
       io.putouts[env] = 0;
     }
   }
-  if (blockIdx.x == 0 && threadIdx.x == 0) io.control->alive = 3u;
 }
 
 __global__ void wildfire_sample_kernel(const FrzWildfireParams p, const FrzWildfireBuffers io, const int B,

@@ -418,6 +418,8 @@ wildfire_tile_kernel(const __grid_constant__ FrzWildfireParams p, const __grid_c
           smem[T.putouts + lane] = uint32_t(n_putout);
           terminated_tile[lane] = terminated;
           truncated_tile[lane] = truncated;
+        } else {  // refresh: the done flags as a reset, a restore or a hand edit left them
+          alive_bits |= (io.terminated[env] ? 0u : 1u) | (io.truncated[env] ? 0u : 2u);
         }
 
         // ------------------------------------------------------------------ update_actions / update_observations

@@ -2,8 +2,12 @@
 
 Environments are independent, so ``parallel_envs`` shards across GPUs with no communication on the step path
 (SURVEY.md section 8e): one process per GPU, each with its own buffers and CUDA graph.  Randomness is keyed by the
-GLOBAL environment index (``env_offset`` + local index), which makes trajectories invariant to the number of shards.
-The statistics record is reduced with one ``all_reduce`` (NCCL over NVLink on GPUs, gloo in the CPU tests).
+GLOBAL environment index (``env_offset`` + local index), so a shard draws the same random numbers as its slice of the
+whole batch.  Its trajectories equal that slice's as long as the reference's two batch-wide conditions agree between
+the shard and the whole batch: "every environment is terminated / truncated" (utils/env.py:212) and "this agent has no
+task in any environment" (wildfire.py:434, rideshare.py:276).  Each shard evaluates them over its own environments, so
+when they differ (one shard entirely terminated, an agent with tasks only in another shard) the shard behaves like the
+reference run on that shard alone.  The statistics record is reduced with one ``all_reduce`` (NCCL over NVLink on GPUs, gloo in the CPU tests).
 """
 from __future__ import annotations
 

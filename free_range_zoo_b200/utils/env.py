@@ -105,7 +105,12 @@ class BatchedAECEnv(ABC):
                 (utils/sql_tap.py; the reference's SQLLogger tables); other connection strings are refused
             single_seeding / buffer_size: accepted and ignored -- randomness is counter-based Philox generated inside
                 the step kernel, keyed by (seed, global env index, step), so there are no generator states to juggle
-            env_offset: global index of this shard's first environment (multi-GPU sharding keeps trajectories invariant)
+            env_offset: global index of this shard's first environment.  Random streams are keyed by the global index,
+                so a shard draws what its environments draw in the whole batch.  The two batch-wide conditions of the
+                reference -- every environment terminated / truncated (utils/env.py:212), an agent without a task in
+                any environment (wildfire.py:434, rideshare.py:276) -- are evaluated over this shard's environments
+                only: a shard equals its slice of the whole batch while those conditions agree, and otherwise equals
+                the reference run on the shard alone
             detach_outputs: return copies instead of views of the in-place updated device buffers
         """
         device = torch.device(device)
@@ -163,12 +168,22 @@ class BatchedAECEnv(ABC):
 
     def load_generator_state_dict(self, state: Dict[str, int]) -> None:
         """Continue the random stream of a checkpoint (reference: ``RandomGenerator.load_state_dict``,
-        utils/random_generator.py:164-176).  Restore the state tensors (``env.state().load(...)`` /
-        ``reset(options={'initial_state': ...})``) and call ``update_actions()`` to re-publish masks and flags."""
+        utils/random_generator.py:164-176).  Restore the state tensors FIRST (``env.state().load(...)`` /
+        ``reset(options={'initial_state': ...})``, the AEC buffers included), then call this: it sets (seed, step),
+        clears recorded faults and re-publishes observations, masks and the batch-wide flags from the restored state.
+
+        The checkpoint must come from an environment with the same ``env_offset``: the random streams are keyed by the
+        global environment index, so another offset would continue on other streams (``ValueError``)."""
+        if int(state['env_offset']) != self.env_offset:
+            raise ValueError(f"the checkpoint was taken with env_offset={int(state['env_offset'])}, this environment has "
+                             f'env_offset={self.env_offset}: its environments would continue on other random streams')
         self._seed_value = int(state['seed'])
         _lib.check(self._lib.frz_control_restore(self._control.data_ptr(), ctypes.c_uint64(int(state['seed'])),
                                                  ctypes.c_uint64(int(state['step'])), self._stream()),
                    'frz_control_restore')
+        self._refresh()
+        self._mid_cycle = False
+        self._rebind_outputs()
 
     # ------------------------------------------------------------------------------------------ properties
 
@@ -272,6 +287,10 @@ class BatchedAECEnv(ABC):
         mask = torch.zeros(self.parallel_envs, dtype=torch.uint8, device=self.device)
         mask[torch.as_tensor(batch_indices, device=self.device, dtype=torch.int64)] = 1
         self._reset_masked(mask)
+        # the observation dictionaries hold gathered copies (other agents' rows, per-agent task views): rebuild them
+        # from the refreshed buffers, as a step does
+        self._mid_cycle = False
+        self._rebind_outputs()
 
     @abstractmethod
     def _reset_masked(self, mask: Optional[torch.Tensor]) -> None:

@@ -415,8 +415,11 @@ const char* frz_last_error(void);
 int frz_control_init(FrzControl* control, uint64_t seed, void* stream);
 /* Restore the random stream of a checkpoint: (seed, step) are all the generator state there is -- every draw is
  * Philox(seed; global env, step, event) -- so this is the engine's load_state_dict (the reference pickles one
- * torch.Generator state per environment: utils/random_generator.py:148-176).  The published flags (alive,
- * agents_with_tasks) are recomputed by the frz_<domain>_refresh the caller runs after restoring the state arrays. */
+ * torch.Generator state per environment: utils/random_generator.py:148-176).  Clears error_word.  The published flags
+ * (alive, agents_with_tasks) are left as they are: restore the state arrays (done flags included), call this, then run
+ * frz_<domain>_refresh, which recomputes both flags from the restored arrays.  frz_<domain>_refresh and
+ * frz_<domain>_reset publish both flags the same way, so a step after a reset or a hand edit of the state sees the done
+ * flags it left. */
 int frz_control_restore(FrzControl* control, uint64_t seed, uint64_t step, void* stream);
 
 /* Size in bytes of the array behind field `field` of Frz<Domain>Buffers (its name as spelled in the struct, e.g.

@@ -95,18 +95,41 @@ class CybersecurityOracle:
         ]
         self.faults = []
 
-    def reset(self):
-        """cybersecurity.py:222-271: actions are pre-filled with -2, so no defender has 'monitored' yet."""
+    STATE_KEYS = ('network_state', 'location', 'presence')
+
+    def reset(self, initial_state: dict | None = None):
+        """cybersecurity.py:222-271 (``initial_state``: network_state [B, N], location [B, D], presence [B, n] instead
+        of the configuration's): actions are pre-filled with -2, so no defender has 'monitored' yet."""
         B = self.B
-        self.network_state = np.tile(self.initial_network, (B, 1))
-        self.location = np.tile(self.initial_location, (B, 1))
-        self.presence = np.tile(self.initial_presence, (B, 1))
+        if initial_state is not None:
+            self.network_state = np.array(initial_state['network_state'], np.int32)
+            self.location = np.array(initial_state['location'], np.int32)
+            self.presence = np.array(initial_state['presence'], bool)
+        else:
+            self.network_state = np.tile(self.initial_network, (B, 1))
+            self.location = np.tile(self.initial_location, (B, 1))
+            self.presence = np.tile(self.initial_presence, (B, 1))
+        self.initial_state = {key: getattr(self, key).copy() for key in self.STATE_KEYS}  # utils/state.py:36-38
         self.last_action_id = np.full((B, self.n_agents), -2, np.int32)
         self.rewards = np.zeros((B, self.n_agents), np.float32)
         self.cumulative_rewards = np.zeros((B, self.n_agents), np.float32)
         self.terminated = np.zeros(B, bool)
         self.truncated = np.zeros(B, bool)
         self.num_moves = np.zeros(B, np.int32)
+        self._publish()
+
+    def reset_batches(self, mask, initial_state: dict | None = None):
+        """utils/env.py:163-189 + cybersecurity.py:274-293: the environments selected by ``mask`` (bool [B]) go back to
+        the saved initial state (``initial_state`` replaces it first when given), their AEC fields are zeroed and their
+        last actions are -2 again (not monitored); then everything is published."""
+        mask = np.asarray(mask, bool)
+        if initial_state is not None:
+            self.initial_state = {key: np.array(initial_state[key], getattr(self, key).dtype) for key in self.STATE_KEYS}
+        for key in self.STATE_KEYS:
+            getattr(self, key)[mask] = self.initial_state[key][mask]
+        self.last_action_id[mask] = -2
+        for key in ('rewards', 'cumulative_rewards', 'terminated', 'truncated', 'num_moves'):
+            getattr(self, key)[mask] = 0
         self._publish()
 
     def _publish(self):

@@ -51,11 +51,20 @@ class RideshareOracle:
 
     # ------------------------------------------------------------------ reset
 
-    def reset(self):
-        """rideshare.py:188-229: agents at their start positions, passengers scheduled for t = 0 enter."""
+    def reset(self, initial_state: dict | None = None):
+        """rideshare.py:188-229: agents at their start positions (or ``initial_state['agents']`` [B, A, 2]), the
+        passenger table empty (or the rows of ``initial_state['passengers']`` [N, 11] whose column 0 is the
+        environment, in their order), then the passengers scheduled for t = 0 enter."""
         B, A = self.B, self.A
-        self.agents = np.tile(self.starts[None], (B, 1, 1)).astype(np.int32)
-        self.tables = [[] for _ in range(B)]  # per env: list of 11-int rows in table order
+        if initial_state is not None:
+            agents = np.array(initial_state['agents'], np.int32)
+            rows = np.asarray(initial_state.get('passengers', np.zeros((0, 11))), np.int64)
+            tables = [[[int(v) for v in row] for row in rows if row[0] == b] for b in range(B)]
+        else:
+            agents, tables = np.tile(self.starts[None], (B, 1, 1)).astype(np.int32), [[] for _ in range(B)]
+        self.initial_state = dict(agents=agents, tables=tables)  # utils/state.py:36-38
+        self.agents = agents.copy()
+        self.tables = [[list(row) for row in table] for table in tables]  # per env: list of 11-int rows in table order
         self.num_moves = np.zeros(B, np.int32)
         self.rewards = np.zeros((B, A), np.float32)
         self.cumulative_rewards = np.zeros((B, A), np.float32)
@@ -64,10 +73,26 @@ class RideshareOracle:
         self._entry(self.num_moves)
         self._publish()
 
-    def _entry(self, timesteps):
+    def reset_batches(self, mask):
+        """utils/env.py:163-189 for the environments selected by ``mask`` (bool [B]): drivers and passenger table back
+        to the saved initial state, AEC fields zeroed, the t = 0 passengers enter again; then everything is published.
+        The reference raises NotImplementedError for a partial rideshare reset (rideshare.py:231-246); this follows
+        the engine's documented intent (include/frz.h, frz_rideshare_reset)."""
+        mask = np.asarray(mask, bool)
+        for b in np.nonzero(mask)[0]:
+            self.agents[b] = self.initial_state['agents'][b]
+            self.tables[b] = [list(row) for row in self.initial_state['tables'][b]]
+        for key in ('rewards', 'cumulative_rewards', 'terminated', 'truncated', 'num_moves'):
+            getattr(self, key)[mask] = 0
+        self._entry(self.num_moves, mask)
+        self._publish()
+
+    def _entry(self, timesteps, mask=None):
         """transitions/passenger_entry.py:25-72: rows whose start time equals the env's timestep (and whose batch
-        is the env or -1) are appended in schedule order."""
+        is the env or -1) are appended in schedule order (only in the environments selected by ``mask``)."""
         for b in range(self.B):
+            if mask is not None and not mask[b]:
+                continue
             for row in self.schedule:
                 if row[0] == timesteps[b] and (row[1] == b or row[1] == -1):
                     self.tables[b].append(

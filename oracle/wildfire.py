@@ -212,11 +212,28 @@ class WildfireOracle:
 
     # ------------------------------------------------------------------ reset
 
+    STATE_KEYS = ('fires', 'intensity', 'fuel', 'suppressants', 'capacity', 'equipment')
+
+    def reset_batches(self, mask, initial_state: dict | None = None):
+        """utils/env.py:163-189 + envs/wildfire/env/wildfire.py:376-397: the environments selected by ``mask`` (bool
+        [B]) go back to the saved initial state (``initial_state`` replaces it first when given) with zeroed AEC fields
+        and counters; then observations and actions are published for the whole batch."""
+        mask = np.asarray(mask, bool)
+        if initial_state is not None:
+            self.initial_state = {key: np.array(initial_state[key]) for key in self.STATE_KEYS}
+        for key in self.STATE_KEYS:
+            getattr(self, key)[mask] = self.initial_state[key][mask]
+        for key in ('rewards', 'cumulative_rewards', 'terminated', 'truncated', 'num_moves', 'num_burnouts', 'burnouts',
+                    'putouts'):
+            getattr(self, key)[mask] = 0
+        self.update_observations()
+        self.update_actions()
+
     def reset(self, initial_state: dict | None = None):
         """utils/env.py:95-160 + envs/wildfire/env/wildfire.py:291-373."""
         B, H, W, A = self.B, self.H, self.W, self.A
         if initial_state is not None:
-            for key in ('fires', 'intensity', 'fuel', 'suppressants', 'capacity', 'equipment'):
+            for key in self.STATE_KEYS:
                 setattr(self, key, np.array(initial_state[key]))
         else:
             self.fires = np.zeros((B, H, W), np.int32)
@@ -229,6 +246,8 @@ class WildfireOracle:
             self.suppressants = np.full((B, A), self.initial[0], np.float32)  # :352-354
             self.capacity = np.full((B, A), self.initial[1], np.float32)
             self.equipment = np.full((B, A), self.initial[2], np.int32)
+        # State.save_initial (utils/state.py:36-38): what reset_batches restores
+        self.initial_state = {key: getattr(self, key).copy() for key in self.STATE_KEYS}
         self.rewards = np.zeros((B, A), np.float32)
         self.cumulative_rewards = np.zeros((B, A), np.float32)
         self.terminated = np.zeros(B, bool)

@@ -130,13 +130,18 @@ def test_two_environments_keep_their_own_pipeline_events():
     assert torch.equal(ra.state().fires, rb.state().fires)
 
 
-@pytest.mark.parametrize('domain,preset,kwargs', [
-    ('wildfire', 'wildfire_large', {}),
-    ('cybersecurity', 'cyber_c3', dict(show_bad_actions=False, partially_observable=True)),
+@pytest.mark.parametrize('domain,preset,kwargs,chunks', [
+    pytest.param('wildfire', 'wildfire_large', {}, None, id='wildfire-wildfire_large-kwargs0'),
+    pytest.param('cybersecurity', 'cyber_c3', dict(show_bad_actions=False, partially_observable=True), None,
+                 id='cybersecurity-cyber_c3-kwargs1'),
+    pytest.param('rideshare', 'rideshare_c2', {}, None, id='rideshare-rideshare_c2'),
+    pytest.param('wildfire', 'wildfire_large', {}, 3, id='wildfire-wildfire_large-step_host'),
+    pytest.param('rideshare', 'rideshare_c2', {}, 3, id='rideshare-rideshare_c2-step_host'),
 ])
-def test_generator_state_restores_a_checkpoint(domain, preset, kwargs):
+def test_generator_state_restores_a_checkpoint(domain, preset, kwargs, chunks):
     """generator_state_dict / load_generator_state_dict (reference: RandomGenerator.state_dict / load_state_dict,
-    utils/random_generator.py:148-176): state tensors + (seed, step) continue a rollout bit for bit."""
+    utils/random_generator.py:148-176): state tensors + (seed, step) continue a rollout bit for bit, through the
+    device step or (``chunks``) the pipelined host step."""
     B = 700
     env = make(domain, preset, kwargs, B, 100)
     env.reset(seed=77)
@@ -158,12 +163,21 @@ def test_generator_state_restores_a_checkpoint(domain, preset, kwargs):
     for name, tensor in checkpoint.items():
         restored._bound[name].copy_(tensor)
     restored.load_generator_state_dict(generator)
-    restored.update_actions()
+    host_actions = torch.empty((B, len(restored.agents), 2), dtype=torch.int32).pin_memory()
     for _ in range(5):
         restored.sample_actions(8)
-        restored.step_all()
+        if chunks is None:
+            restored.step_all()
+        else:
+            host_actions.copy_(restored._actions)
+            torch.cuda.synchronize()
+            restored.step_host(host_actions, chunks)
     for name, tensor in want.items():
-        assert torch.equal(restored._bound[name], tensor), name
+        if domain == 'rideshare' and name == 'passengers':  # rows beyond the count are undefined
+            valid = torch.arange(restored._capacity, device='cuda')[None, :] < restored.environment_task_count[:, None]
+            assert torch.equal(restored._bound[name][valid], tensor[valid]), name
+        else:
+            assert torch.equal(restored._bound[name], tensor), name
 
 
 def test_capture_graph_does_not_advance_the_environment():
