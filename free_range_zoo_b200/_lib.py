@@ -160,6 +160,23 @@ class ObsDownload(C.Structure):
                 ('mask_groups', C.c_int32)]
 
 
+class AutoresetRow(C.Structure):
+    """FrzAutoresetRow (include/frz_autoreset.h): one per-environment array a restart restores (src NULL = zeros)."""
+    _fields_ = [('dst', C.c_void_p), ('src', C.c_void_p), ('bytes', C.c_int64)]
+
+
+AUTORESET_MAX_ROWS = 32
+
+
+class Autoreset(C.Structure):
+    """FrzAutoreset (include/frz_autoreset.h): flags, episode statistics, scratch and rows of the same-step autoreset."""
+    _fields_ = [(name, C.c_void_p) for name in (
+        'terminated', 'truncated', 'step_terminated', 'step_truncated', 'done', 'cumulative_rewards', 'episode_return',
+        'num_moves', 'episode_length', 'agent_task_count', 'reset_agent_task_count', 'control', 'finished',
+        'finished_count', 'scratch')] + [('rows', C.POINTER(AutoresetRow)), ('row_count', C.c_int32),
+                                         ('num_agents', C.c_int32)]
+
+
 OBS_DENSE, OBS_ROWS, OBS_MASK_BITS = 0, 1, 2
 OBS_I32, OBS_I16, OBS_I8, OBS_U8, OBS_F32 = 0, 1, 2, 3, 4
 HOST_ACTIONS_I32, HOST_ACTIONS_I16, HOST_ACTIONS_I8 = 0, 1, 2
@@ -207,6 +224,7 @@ def library() -> C.CDLL:
     lib.frz_gather_live_rows.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(GatherArray), C.c_int32,
                                          C.c_void_p]
     lib.frz_observe_compact.argtypes = [C.POINTER(ObsDownload), C.c_int32, C.c_void_p]
+    lib.frz_autoreset.argtypes = [C.POINTER(Autoreset), C.c_int32, C.c_void_p]
     if lib.frz_version() != ABI_VERSION:
         raise RuntimeError(f'libfrz.so ABI version {lib.frz_version()} != {ABI_VERSION}; rebuild the library')
     lib.frz_control_restore.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p]

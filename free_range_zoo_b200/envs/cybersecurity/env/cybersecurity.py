@@ -19,7 +19,7 @@ from free_range_zoo_b200.envs.cybersecurity.env.structures.state import Cybersec
 from free_range_zoo_b200.utils.containers import LazyDict, ObservationDict, jagged_indices_from_mask
 from free_range_zoo_b200.utils.conversions import batched_aec_to_batched_parallel
 from free_range_zoo_b200.utils import compact
-from free_range_zoo_b200.utils.env import BatchedAECEnv
+from free_range_zoo_b200.utils.env import AutoresetRows, BatchedAECEnv
 from free_range_zoo_b200.utils.spaces import BatchedActionSpace, Space
 
 
@@ -202,6 +202,7 @@ class raw_env(BatchedAECEnv):
                                       .unsqueeze(0).expand_as(self._init_presence))
         self._actions.fill_(-2)  # cybersecurity.py:233-236
         self._reset_masked(None)
+        self._snapshot_reset()
         self._rebind_outputs()
         if self.log_directory is not None:
             self._log_environment(reset=True)
@@ -235,6 +236,20 @@ class raw_env(BatchedAECEnv):
         """cybersecurity.py:580-584: the adjacency matrix on every row."""
         adjacency = str(torch.as_tensor(self.network_config.adj_matrix).int().tolist())
         return {'adj_matrix': [adjacency] * self.parallel_envs}
+
+    @classmethod
+    def _autoreset_rows(cls) -> AutoresetRows:
+        """A restart as cyber_restore_kernel + refresh: state from init_*, the refresh's outputs from the snapshot,
+        AEC fields and ``monitored`` (the last actions are -2 again) zeroed; rewards written by every step.  The domain
+        has no per-agent skip: agents_with_tasks stays 0."""
+        return AutoresetRows(
+            init={'network_state': 'init_network_state', 'location': 'init_location', 'presence': 'init_presence'},
+            snapshot=('env_task_count', 'agent_task_count', 'attacker_self', 'defender_self', 'task_obs'),
+            zero=('monitored', 'cumulative_rewards', 'terminated', 'truncated', 'num_moves'),
+            overwritten=('rewards', ),
+            static=('init_network_state', 'init_location', 'init_presence', 'actions', 'score_lut', 'control',
+                    'network_uniforms', 'agent_uniforms'),
+            agents_with_tasks=False)
 
     # ------------------------------------------------------------------------------------------ step
 

@@ -19,7 +19,7 @@ from free_range_zoo_b200.utils.containers import (LazyDict, ObservationDict, jag
                                                   jagged_rows_from_mask)
 from free_range_zoo_b200.utils.conversions import batched_aec_to_batched_parallel
 from free_range_zoo_b200.utils import compact
-from free_range_zoo_b200.utils.env import BatchedAECEnv
+from free_range_zoo_b200.utils.env import AutoresetRows, BatchedAECEnv
 from free_range_zoo_b200.utils.spaces import BatchedActionSpace, Space
 
 
@@ -185,6 +185,7 @@ class raw_env(BatchedAECEnv):
             starts = torch.as_tensor(self.agent_config.start_positions, dtype=torch.int32).to(dev)
             self._init_agents.copy_(starts.unsqueeze(0).expand_as(self._init_agents))
         self._reset_masked(None)
+        self._snapshot_reset()
         self._rebind_outputs()
         if self.log_directory is not None:
             self._log_environment(reset=True)
@@ -192,6 +193,19 @@ class raw_env(BatchedAECEnv):
     def _reset_masked(self, mask: Optional[torch.Tensor]) -> None:
         _lib.check(self._lib.frz_rideshare_reset(ctypes.byref(self._params), ctypes.byref(self._io), self.parallel_envs,
                                                  _lib.pointer(mask), self._stream()), 'frz_rideshare_reset')
+
+    @classmethod
+    def _autoreset_rows(cls) -> AutoresetRows:
+        """A restart as rideshare_restore_kernel + the t = 0 entry: drivers from init_agents; the passenger table and its
+        count after the entry, like the observations, masks and counts, from the snapshot (the t = 0 entry depends on
+        the schedule and the environment's index only); AEC fields zeroed; rewards written by every step."""
+        return AutoresetRows(
+            init={'agents': 'init_agents'},
+            snapshot=('passengers', 'env_task_count', 'agent_task_count', 'task_mask', 'self_obs', 'task_obs'),
+            zero=('cumulative_rewards', 'terminated', 'truncated', 'num_moves'),
+            overwritten=('rewards', ),
+            static=('init_agents', 'init_passengers', 'init_count', 'schedule', 'schedule_index', 'actions', 'control'),
+            agents_with_tasks=True)
 
     # ------------------------------------------------------------------------------------------ step
 

@@ -19,7 +19,7 @@ from free_range_zoo_b200.utils.containers import (LazyDict, ObservationDict, jag
                                                   jagged_indices_from_mask)
 from free_range_zoo_b200.utils.conversions import batched_aec_to_batched_parallel
 from free_range_zoo_b200.utils import compact
-from free_range_zoo_b200.utils.env import BatchedAECEnv
+from free_range_zoo_b200.utils.env import AutoresetRows, BatchedAECEnv
 from free_range_zoo_b200.utils.spaces import BatchedActionSpace, Space
 
 
@@ -274,6 +274,7 @@ class raw_env(BatchedAECEnv):
         self.fire_reduction_power = ac.fire_reduction_power
         self.suppressant_states = ac.suppressant_states
         self._reset_masked(None)
+        self._snapshot_reset()
         self.infos = dict({agent: {} for agent in self.agents}, burnouts=self._burnouts, putouts=self._putouts)
         self._rebind_outputs()
         if self.log_directory is not None:
@@ -283,6 +284,22 @@ class raw_env(BatchedAECEnv):
         """frz_wildfire_reset: restore initial rows, zero AEC fields (+ num_burnouts, wildfire.py:393), refresh."""
         _lib.check(self._lib.frz_wildfire_reset(ctypes.byref(self._params), ctypes.byref(self._io), self.parallel_envs,
                                                 _lib.pointer(mask), self._stream()), 'frz_wildfire_reset')
+
+    @classmethod
+    def _autoreset_rows(cls) -> AutoresetRows:
+        """A restart as wildfire_restore_kernel + refresh: state from init_*, the refresh's outputs from the snapshot,
+        AEC fields and the burn-out total zeroed; rewards and the per-step burn-out / put-out counts are written for
+        every environment by every step."""
+        state = ('fires', 'intensity', 'fuel', 'suppressants', 'capacity', 'equipment')
+        return AutoresetRows(
+            init={name: f'init_{name}' for name in state},
+            snapshot=('action_mask', 'self_obs', 'task_obs', 'env_task_count', 'agent_task_count'),
+            zero=('cumulative_rewards', 'terminated', 'truncated', 'num_moves', 'num_burnouts'),
+            overwritten=('rewards', 'burnouts', 'putouts'),
+            static=tuple(f'init_{name}' for name in state) + (
+                'actions', 'cell_reward', 'cell_ignition', 'range_mask', 'cell_agents', 'control', 'field_uniforms',
+                'agent_uniforms'),
+            agents_with_tasks=True)
 
     # ------------------------------------------------------------------------------------------ step
 

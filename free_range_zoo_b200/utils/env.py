@@ -22,7 +22,7 @@ from __future__ import annotations
 import ctypes
 import math
 from abc import ABC, abstractmethod
-from typing import Any, Dict, List, Optional, Tuple
+from typing import Any, Dict, List, NamedTuple, Optional, Tuple
 
 import torch
 
@@ -35,6 +35,17 @@ from free_range_zoo_b200.utils.selector import AgentSelector
 
 # most slices ``step_host`` cuts a batch into by default (measured on B200, profiles/README.md)
 HOST_STEP_MAX_DEFAULT_CHUNKS = 5
+
+
+class AutoresetRows(NamedTuple):
+    """What a restart does with each per-environment buffer a domain binds (``_bound`` keys).  Every key is in exactly
+    one of the five groups, so a buffer added later needs a decision (tests/test_autoreset.py)."""
+    init: Dict[str, str]  # state restored from its initial copy: {buffer: its init_* buffer}
+    snapshot: Tuple[str, ...]  # outputs of the reset's refresh, restored from the snapshot taken at reset()
+    zero: Tuple[str, ...]  # AEC fields the next step reads, zeroed as the domain's reset kernel zeroes them
+    overwritten: Tuple[str, ...]  # written for every environment by every step: kept as the finishing step wrote them
+    static: Tuple[str, ...]  # not changed by a restart: init_* copies, inputs, configuration tables, the control block
+    agents_with_tasks: bool  # whether the domain publishes FrzControl.agents_with_tasks (a refresh publishes 0 otherwise)
 
 
 class _DeviceBound:
@@ -91,6 +102,7 @@ class BatchedAECEnv(ABC):
         override_initialization_check: bool = False,
         env_offset: int = 0,
         detach_outputs: bool = False,
+        autoreset: bool = False,
         **kwargs,
     ):
         """
@@ -112,6 +124,19 @@ class BatchedAECEnv(ABC):
                 only: a shard equals its slice of the whole batch while those conditions agree, and otherwise equals
                 the reference run on the shard alone
             detach_outputs: return copies instead of views of the in-place updated device buffers
+            autoreset: restart every environment that is terminated or truncated at the end of the step that finished
+                it ("same-step" autoreset), on the device and in the same stream / CUDA graph as the step: ``step``,
+                ``step_all``, the Parallel ``step``, ``step_host`` and every step of a ``capture_graph(steps=K)`` replay.
+                Afterwards state, observations, masks, counts and the batch-wide flags are what ``reset_batches`` of the
+                finished environments leaves.  What the step returns (rewards, terminations, truncations, infos) is what
+                the finishing step produced; ``terminated`` / ``truncated`` / ``finished`` / ``terminations`` /
+                ``truncations`` read copies of the step's done flags ("the episode ended at the last step") and
+                ``episode_statistics`` gives each finished episode's return and length.  Restarted environments keep
+                drawing random numbers with the global step counter, as after ``reset_batches``.  The final observation
+                of a finished episode is not kept: the observations after the step are the restarted environment's.
+                Every full ``reset()`` snapshots the per-environment outputs of its refresh (observations, masks,
+                counts, rideshare's passenger table), which a restart copies back: about 2.8 KB per environment at
+                wildfire C4 (184 MB at 65 536 environments).  Not available with a ``log_directory``.
         """
         device = torch.device(device)
         if device.type != 'cuda':
@@ -133,6 +158,10 @@ class BatchedAECEnv(ABC):
         self.logger = None
         self.env_offset = int(env_offset)
         self.detach_outputs = detach_outputs
+        self.autoreset = bool(autoreset)
+        if self.autoreset and log_directory is not None:
+            raise ValueError('autoreset restarts environments on the device inside the step, which the logging tap does not '
+                             'record; autoreset=True needs log_directory=None')
 
         if configuration is not None:
             self.config = configuration
@@ -201,12 +230,30 @@ class BatchedAECEnv(ABC):
 
     @property
     def terminated(self) -> torch.Tensor:
-        """bool [B]; every agent of an environment terminates together (reference utils/env.py:341-349)."""
+        """bool [B]; every agent of an environment terminates together (reference utils/env.py:341-349).  With
+        ``autoreset`` a copy of what the last step produced (the live flags of a restarted environment are clear)."""
+        if self.autoreset:
+            return self._autoreset_flags[1].view(torch.bool)
         return self._terminated.view(torch.bool)
 
     @property
     def truncated(self) -> torch.Tensor:
+        if self.autoreset:
+            return self._autoreset_flags[2].view(torch.bool)
         return self._truncated.view(torch.bool)
+
+    @property
+    def episode_statistics(self) -> Dict[str, torch.Tensor]:
+        """The episodes the last step finished (``autoreset=True`` only), device tensors overwritten by the next step:
+        ``done`` / ``terminated`` / ``truncated`` bool [B], ``return`` f32 [B, A] (the cumulative reward of the episode)
+        and ``length`` int32 [B] (its number of steps).  ``return`` and ``length`` are defined only where ``done`` is
+        set; elsewhere they hold an earlier episode's values or zeros, so select with ``done`` before reducing (e.g.
+        ``distributed.episode_statistics(s['return'][s['done']], ...)``)."""
+        if not self.autoreset:
+            raise RuntimeError('episode_statistics is recorded by the autoreset: construct the environment with autoreset=True')
+        flags = self._autoreset_flags.view(torch.bool)
+        return {'done': flags[0], 'terminated': flags[1], 'truncated': flags[2], 'return': self._episode_return,
+                'length': self._episode_length}
 
     @property
     def finished(self) -> torch.Tensor:
@@ -239,6 +286,13 @@ class BatchedAECEnv(ABC):
         self.environment_task_count = torch.zeros(B, dtype=torch.int32, device=dev)
         self._agent_task_count = torch.zeros((B, A), dtype=torch.int32, device=dev)
         self._zero_rewards = torch.zeros(B, dtype=torch.float32, device=dev)
+        if self.autoreset:
+            self._autoreset_flags = torch.zeros((3, B), dtype=torch.uint8, device=dev)  # done, terminated, truncated
+            self._episode_return = torch.zeros((B, A), dtype=torch.float32, device=dev)
+            self._episode_length = torch.zeros(B, dtype=torch.int32, device=dev)
+            self._autoreset_list = torch.zeros(B, dtype=torch.int32, device=dev)
+            self._autoreset_count = torch.zeros(1, dtype=torch.int32, device=dev)
+            self._autoreset_scratch = torch.zeros(2, dtype=torch.int32, device=dev)  # left zero by every launch
 
     def _stream(self) -> ctypes.c_void_p:
         return _lib.stream_handle(self.device)
@@ -287,6 +341,8 @@ class BatchedAECEnv(ABC):
         mask = torch.zeros(self.parallel_envs, dtype=torch.uint8, device=self.device)
         mask[torch.as_tensor(batch_indices, device=self.device, dtype=torch.int64)] = 1
         self._reset_masked(mask)
+        if self.autoreset:  # a restarted environment's episode did not end at the last step
+            self._autoreset_flags.masked_fill_(mask.bool(), 0)
         # the observation dictionaries hold gathered copies (other agents' rows, per-agent task views): rebuild them
         # from the refreshed buffers, as a step does
         self._mid_cycle = False
@@ -295,6 +351,53 @@ class BatchedAECEnv(ABC):
     @abstractmethod
     def _reset_masked(self, mask: Optional[torch.Tensor]) -> None:
         """Launch the domain's reset kernel for the environments selected by ``mask`` (uint8 [B]; None = all)."""
+
+    # ------------------------------------------------------------------------------------------ autoreset
+
+    @classmethod
+    def _autoreset_rows(cls) -> AutoresetRows:
+        """How a restart treats each buffer of ``_bound``.  Domain hook."""
+        raise NotImplementedError
+
+    def _snapshot_reset(self) -> None:
+        """After a full reset: with ``autoreset``, keep the outputs of the reset's refresh, which are what a restart
+        restores, and describe the rows of ``frz_autoreset`` (include/frz_autoreset.h)."""
+        if not self.autoreset:
+            return
+        B, rows, bound = self.parallel_envs, self._autoreset_rows(), self._bound
+        if getattr(self, '_reset_snapshot', None) is None:
+            self._reset_snapshot = {name: torch.empty_like(bound[name]) for name in rows.snapshot}
+        for name, tensor in self._reset_snapshot.items():
+            tensor.copy_(bound[name])
+        self._autoreset_flags.zero_()
+        pairs = ([(bound[dst], bound[src]) for dst, src in rows.init.items()] +
+                 [(bound[name], self._reset_snapshot[name]) for name in rows.snapshot] +
+                 [(bound[name], None) for name in rows.zero])
+        table = (_lib.AutoresetRow * len(pairs))()
+        for at, (dst, src) in enumerate(pairs):
+            assert dst.shape[0] == B and dst.is_contiguous() and (src is None or src.shape == dst.shape)
+            table[at].dst, table[at].src = dst.data_ptr(), _lib.pointer(src)
+            table[at].bytes = dst.numel() * dst.element_size() // B
+        block = _lib.Autoreset()
+        block.terminated, block.truncated = self._terminated.data_ptr(), self._truncated.data_ptr()
+        block.done, block.step_terminated, block.step_truncated = (row.data_ptr() for row in self._autoreset_flags)
+        block.cumulative_rewards, block.episode_return = self._cumulative.data_ptr(), self._episode_return.data_ptr()
+        block.num_moves, block.episode_length = self.num_moves.data_ptr(), self._episode_length.data_ptr()
+        if rows.agents_with_tasks:
+            block.agent_task_count = self._agent_task_count.data_ptr()
+            block.reset_agent_task_count = self._reset_snapshot['agent_task_count'].data_ptr()
+        block.control = self._control.data_ptr()
+        block.finished, block.finished_count = self._autoreset_list.data_ptr(), self._autoreset_count.data_ptr()
+        block.scratch = self._autoreset_scratch.data_ptr()
+        block.rows, block.row_count = table, len(pairs)
+        block.num_agents = self._cumulative.shape[1]
+        self._autoreset_block = (block, table)  # (the table must outlive the block that points at it)
+
+    def _autoreset_launch(self) -> None:
+        """Restart the environments the step just finished (two launches on the current stream; no host read)."""
+        if self.autoreset:
+            _lib.check(self._lib.frz_autoreset(ctypes.byref(self._autoreset_block[0]), self.parallel_envs, self._stream()),
+                       'frz_autoreset')
 
     # ------------------------------------------------------------------------------------------ step
 
@@ -529,6 +632,10 @@ class BatchedAECEnv(ABC):
         main.wait_stream(current)
         _lib.check(self._host_entry()(ctypes.byref(self._params), ctypes.byref(self._io), B,
                                       ctypes.byref(state['block']), ctypes.c_void_p(main.cuda_stream)), 'step_host')
+        # (every slice's reward download and the done-flag download are on `main` before this point, so the host
+        # results are the finishing step's)
+        with torch.cuda.stream(main):
+            self._autoreset_launch()
         current.wait_stream(main)  # later work on the caller's stream sees the stepped state
         # host-side bookkeeping while the device works; the views do not depend on the data
         self._mid_cycle = False
@@ -552,6 +659,7 @@ class BatchedAECEnv(ABC):
 
     def _advance(self) -> None:
         _, _, infos = self.step_environment()
+        self._autoreset_launch()
         self.infos = infos
         self._mid_cycle = False
         self._rebind_outputs()
@@ -677,7 +785,7 @@ class BatchedAECEnv(ABC):
     # ------------------------------------------------------------------------------------------ CUDA graph
 
     def capture_graph(self, sample: bool = False, sampler_seed: int = 2026, steps: int = 1) -> None:
-        """Capture ``steps`` x ``[sample_actions ->] step`` in a CUDA graph; ``replay()`` then costs one graph launch
+        """Capture ``steps`` x ``[sample_actions ->] step [-> autoreset]`` in a CUDA graph; ``replay()`` then costs one graph launch
         per ``steps`` environment steps (small batches are bound by launch latency: several steps per launch keep the
         kernels back to back).  Kernel arguments are pointer-stable and the step counter lives on the device, so the
         graph needs no updates.  Capturing leaves the environment where it was (the warm-up launch is undone).  Replays
@@ -690,16 +798,21 @@ class BatchedAECEnv(ABC):
         # so capturing does not advance the environment
         saved = {name: tensor.clone() for name, tensor in self._bound.items()
                  if tensor is not None and not name.startswith('init_')}
+        autoreset = [self._autoreset_flags, self._episode_return, self._episode_length] if self.autoreset else []
+        saved_autoreset = [tensor.clone() for tensor in autoreset]
         side = torch.cuda.Stream(self.device)
         side.wait_stream(torch.cuda.current_stream(self.device))
         with torch.cuda.stream(side):
             if sample:
                 self.sample_actions(sampler_seed)
             self.step_environment()
+            self._autoreset_launch()
         torch.cuda.current_stream(self.device).wait_stream(side)
         torch.cuda.synchronize(self.device)
         for name, tensor in saved.items():
             self._bound[name].copy_(tensor)
+        for tensor, copy in zip(autoreset, saved_autoreset):
+            tensor.copy_(copy)
         del saved
         torch.cuda.synchronize(self.device)
         graph = torch.cuda.CUDAGraph()
@@ -708,6 +821,7 @@ class BatchedAECEnv(ABC):
                 if sample:
                     self.sample_actions(sampler_seed)
                 self.step_environment()
+                self._autoreset_launch()
         self._graph = graph
 
     def replay(self) -> None:
