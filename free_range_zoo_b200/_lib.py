@@ -161,8 +161,9 @@ class ObsDownload(C.Structure):
 
 
 class AutoresetRow(C.Structure):
-    """FrzAutoresetRow (include/frz_autoreset.h): one per-environment array a restart restores (src NULL = zeros)."""
-    _fields_ = [('dst', C.c_void_p), ('src', C.c_void_p), ('bytes', C.c_int64)]
+    """FrzAutoresetRow (include/frz_autoreset.h): one per-environment array a restart restores (src NULL = zeros),
+    its pre-restart bytes copied to ``keep`` first unless that is NULL."""
+    _fields_ = [('dst', C.c_void_p), ('src', C.c_void_p), ('bytes', C.c_int64), ('keep', C.c_void_p)]
 
 
 AUTORESET_MAX_ROWS = 32

@@ -10,6 +10,7 @@
 //   autoreset_restore  persistent grid over (row, group of listed environments) warp items: a row gets as many lanes per
 //                      environment as it has words (up to 32), so one warp restores 32 one-word rows or one long row;
 //                      16-byte words where the addresses and the row size allow.  No atomics, nothing to publish.
+//                      A row with a `keep` array has each word's old value stored there before the word is restored.
 // Work is proportional to the number of finished environments, plus the scan's read of the flags and, for the
 // environments that go on, their per-agent task counts.
 #include "frz_autoreset.h"
@@ -80,24 +81,36 @@ __global__ void __launch_bounds__(kScanThreads) autoreset_scan_kernel(const FrzA
   }
 }
 
-// the `rank`-th of `threads` threads copies its share of one row of `bytes` bytes in words of type Word
-template <class Word>
-__device__ __forceinline__ void copy_words(char* dst, const char* src, size_t bytes, int rank, int threads) {
+// the `rank`-th of `threads` threads copies its share of one row of `bytes` bytes in words of type Word; with kKeep it
+// first stores each word's current value to `keep` (the same thread loads and overwrites the same address: no ordering)
+template <class Word, bool kKeep>
+__device__ __forceinline__ void copy_words(char* dst, const char* src, char* keep, size_t bytes, int rank, int threads) {
   const size_t words = bytes / sizeof(Word);
-  for (size_t i = rank; i < words; i += threads)
+  for (size_t i = rank; i < words; i += threads) {
+    if (kKeep) reinterpret_cast<Word*>(keep)[i] = reinterpret_cast<const Word*>(dst)[i];
     reinterpret_cast<Word*>(dst)[i] = src != nullptr ? reinterpret_cast<const Word*>(src)[i] : Word{};
+  }
+}
+
+template <bool kKeep>
+__device__ __forceinline__ void restore_words(char* dst, const char* src, char* keep, size_t bytes, int word, int rank,
+                                              int threads) {
+  switch (word) {
+    case 16: copy_words<uint4, kKeep>(dst, src, keep, bytes, rank, threads); break;
+    case 8: copy_words<uint2, kKeep>(dst, src, keep, bytes, rank, threads); break;
+    case 4: copy_words<uint32_t, kKeep>(dst, src, keep, bytes, rank, threads); break;
+    default: copy_words<uint8_t, kKeep>(dst, src, keep, bytes, rank, threads); break;
+  }
 }
 
 __device__ __forceinline__ void restore_row(const FrzAutoresetRow& row, int word, int env, int rank, int threads) {
   const size_t bytes = size_t(row.bytes);
   char* dst = static_cast<char*>(row.dst) + size_t(env) * bytes;
   const char* src = row.src != nullptr ? static_cast<const char*>(row.src) + size_t(env) * bytes : nullptr;
-  switch (word) {
-    case 16: copy_words<uint4>(dst, src, bytes, rank, threads); break;
-    case 8: copy_words<uint2>(dst, src, bytes, rank, threads); break;
-    case 4: copy_words<uint32_t>(dst, src, bytes, rank, threads); break;
-    default: copy_words<uint8_t>(dst, src, bytes, rank, threads); break;
-  }
+  if (row.keep != nullptr)
+    restore_words<true>(dst, src, static_cast<char*>(row.keep) + size_t(env) * bytes, bytes, word, rank, threads);
+  else
+    restore_words<false>(dst, src, nullptr, bytes, word, rank, threads);
 }
 
 __global__ void __launch_bounds__(kRestoreThreads) autoreset_restore_kernel(const FrzAutoreset a, const RowTable rows) {
@@ -156,7 +169,7 @@ extern "C" int frz_autoreset(const FrzAutoreset* autoreset, int32_t parallel_env
       return FRZ_ERR_SHAPE;
     }
     const uintptr_t alignment = reinterpret_cast<uintptr_t>(row.dst) | reinterpret_cast<uintptr_t>(row.src) |
-                                uintptr_t(row.bytes);
+                                reinterpret_cast<uintptr_t>(row.keep) | uintptr_t(row.bytes);
     const int word = (alignment & 15u) == 0 ? 16 : (alignment & 7u) == 0 ? 8 : (alignment & 3u) == 0 ? 4 : 1;
     const int64_t words = row.bytes / word;
     int lanes = 1;

@@ -249,7 +249,8 @@ class raw_env(BatchedAECEnv):
             overwritten=('rewards', ),
             static=('init_network_state', 'init_location', 'init_presence', 'actions', 'score_lut', 'control',
                     'network_uniforms', 'agent_uniforms'),
-            agents_with_tasks=False)
+            agents_with_tasks=False,
+            final=('attacker_self', 'defender_self', 'task_obs', 'monitored', 'env_task_count', 'agent_task_count'))
 
     # ------------------------------------------------------------------------------------------ step
 
@@ -265,23 +266,25 @@ class raw_env(BatchedAECEnv):
         _lib.check(self._lib.frz_cyber_refresh(ctypes.byref(self._params), ctypes.byref(self._io), self.parallel_envs,
                                                self._stream()), 'frz_cyber_refresh')
 
-    def _observation_download(self):
+    def _observation_download(self, buffers=None):
         """Host-side observation download (``gather_observations``): every environment always has all N subnetworks as
         tasks, so everything is dense."""
-        dense = dict(attacker_self=self._attacker_self, defender_self=self._defender_self, task_obs=self._task_obs,
-                     monitored=self._monitored, agent_task_count=self._agent_task_count)
+        b = self._observation_buffers() if buffers is None else buffers
+        dense = dict(attacker_self=b['attacker_self'], defender_self=b['defender_self'], task_obs=b['task_obs'],
+                     monitored=b['monitored'], agent_task_count=b['agent_task_count'])
         return dense, {}
 
-    def _compact_schema(self):
+    def _compact_schema(self, buffers=None):
         """Compact download (utils/compact.py): task rows and counts narrowed; the float arrays and ``monitored`` as
         they are.  Every environment has all subnetworks as tasks, so everything is dense."""
+        b = self._observation_buffers() if buffers is None else buffers
         bounds = compact_bounds(self._params)
         return compact.Schema(capacity=int(self._params.num_nodes), arrays=[
-            compact.dense('attacker_self', self._attacker_self),
-            compact.dense('defender_self', self._defender_self),
-            compact.dense('task_obs', self._task_obs, bound=bounds['task_obs']),
-            compact.dense('monitored', self._monitored),
-            compact.dense('agent_task_count', self._agent_task_count, bound=bounds['agent_task_count']),
+            compact.dense('attacker_self', b['attacker_self']),
+            compact.dense('defender_self', b['defender_self']),
+            compact.dense('task_obs', b['task_obs'], bound=bounds['task_obs']),
+            compact.dense('monitored', b['monitored']),
+            compact.dense('agent_task_count', b['agent_task_count'], bound=bounds['agent_task_count']),
         ])
 
     def update_actions(self) -> None:
@@ -313,12 +316,13 @@ class raw_env(BatchedAECEnv):
         """int64 [B, N, 2] = (state, criticality), like the reference (cybersecurity.py:488)."""
         return self._task_obs.to(torch.int64)
 
-    def _tasks_for(self, agent: str):
+    def _tasks_for(self, agent: str, buffers):
         """A defender under partial observability sees -100 unless its last action was monitor (:497,510-511)."""
+        task_obs, monitored = buffers['task_obs'], buffers['monitored']
         if agent in self.defender_name_mapping and self.partially_observable:
             d = self.defender_name_mapping[agent]
-            return lambda: torch.where(self._monitored[:, d].view(-1, 1, 1) != 0, self._task_obs, -100).to(torch.int64)
-        return lambda: self._task_obs.to(torch.int64)
+            return lambda: torch.where(monitored[:, d].view(-1, 1, 1) != 0, task_obs, -100).to(torch.int64)
+        return lambda: task_obs.to(torch.int64)
 
     def _other_indices(self, count: int, index: int) -> torch.Tensor:
         """Indices of the other agents of the same kind (device tensors built once: this runs every step)."""
@@ -333,26 +337,31 @@ class raw_env(BatchedAECEnv):
             self._node_index_cache = torch.arange(self._n_nodes, device=self.device).unsqueeze(0)
         return self._node_index_cache
 
-    def update_observation_views(self) -> None:
-        B, N = self.parallel_envs, self._n_nodes
-        self.observations = {}
+    def _observation_views(self, buffers) -> Dict[str, ObservationDict]:
+        B = self.parallel_envs
+        views = {}
         for agent in self.agents:
             if agent in self.attacker_name_mapping:
-                index, table, columns, count = (self.attacker_name_mapping[agent], self._attacker_self,
+                index, table, columns, count = (self.attacker_name_mapping[agent], buffers['attacker_self'],
                                                 self._attacker_columns, self._n_att)
             else:
-                index, table, columns, count = (self.defender_name_mapping[agent], self._defender_self,
+                index, table, columns, count = (self.defender_name_mapping[agent], buffers['defender_self'],
                                                 self._defender_columns, self._n_def)
             others = self._other_indices(count, index)
-            self.observations[agent] = ObservationDict(
+            views[agent] = ObservationDict(
                 {
                     'self': table[:, index],
                     'others': (lambda t=table, o=others, c=columns: t[:, o][:, :, c]),
-                    'tasks': self._tasks_for(agent),
+                    'tasks': self._tasks_for(agent, buffers),
                 },
                 batch_size=[B],
                 device=self.device,
             )
+        return views
+
+    def update_observation_views(self) -> None:
+        B = self.parallel_envs
+        self.observations = self._observation_views(self._observation_buffers())
         nodes = self._node_indices()
         self.agent_action_mapping = LazyDict({
             a: (lambda i=i: jagged_indices_from_mask(nodes < self._agent_task_count[:, i].unsqueeze(1)))

@@ -205,7 +205,8 @@ class raw_env(BatchedAECEnv):
             zero=('cumulative_rewards', 'terminated', 'truncated', 'num_moves'),
             overwritten=('rewards', ),
             static=('init_agents', 'init_passengers', 'init_count', 'schedule', 'schedule_index', 'actions', 'control'),
-            agents_with_tasks=True)
+            agents_with_tasks=True,
+            final=('self_obs', 'task_obs', 'task_mask', 'env_task_count', 'agent_task_count'))
 
     # ------------------------------------------------------------------------------------------ step
 
@@ -221,22 +222,24 @@ class raw_env(BatchedAECEnv):
         _lib.check(self._lib.frz_rideshare_refresh(ctypes.byref(self._params), ctypes.byref(self._io),
                                                    self.parallel_envs, self._stream()), 'frz_rideshare_refresh')
 
-    def _observation_download(self):
+    def _observation_download(self, buffers=None):
         """Host-side observation download (``gather_observations``): self observations and per-driver task counts whole,
         the live rows of the task observations and of every driver's task-mask row packed."""
-        dense = dict(self_obs=self._self_obs, agent_task_count=self._agent_task_count)
-        ragged = dict(task_obs=(self._task_obs, 1), task_mask=(self._task_mask, len(self.possible_agents)))
+        b = self._observation_buffers() if buffers is None else buffers
+        dense = dict(self_obs=b['self_obs'], agent_task_count=b['agent_task_count'])
+        ragged = dict(task_obs=(b['task_obs'], 1), task_mask=(b['task_mask'], len(self.possible_agents)))
         return dense, ragged
 
-    def _compact_schema(self):
+    def _compact_schema(self, buffers=None):
         """Compact download (utils/compact.py): live task rows, the task mask as bits, self observations and counts."""
+        b = self._observation_buffers() if buffers is None else buffers
         A = len(self.possible_agents)
         bounds = compact_bounds(self.config, self._params, self.max_steps)
         return compact.Schema(capacity=self._capacity, mask_groups=A, arrays=[
-            compact.rows('task_obs', self._task_obs, bound=bounds['task_obs']),
-            compact.mask('task_mask', self._task_mask, groups=A),
-            compact.dense('self_obs', self._self_obs, bound=bounds['self_obs']),
-            compact.dense('agent_task_count', self._agent_task_count, bound=bounds['agent_task_count']),
+            compact.rows('task_obs', b['task_obs'], bound=bounds['task_obs']),
+            compact.mask('task_mask', b['task_mask'], groups=A),
+            compact.dense('self_obs', b['self_obs'], bound=bounds['self_obs']),
+            compact.dense('agent_task_count', b['agent_task_count'], bound=bounds['agent_task_count']),
         ])
 
     def update_actions(self) -> None:
@@ -287,22 +290,27 @@ class raw_env(BatchedAECEnv):
         rows = torch.arange(self._capacity, device=self.device).unsqueeze(0) < self.environment_task_count.unsqueeze(1)
         return jagged_rows_from_mask(self._task_obs, rows)
 
-    def update_observation_views(self) -> None:
+    def _observation_views(self, buffers) -> Dict[str, ObservationDict]:
         B = self.parallel_envs
-        self.observations = {}
+        self_obs, task_obs, task_mask = buffers['self_obs'], buffers['task_obs'], buffers['task_mask'].view(torch.bool)
+        views = {}
         for agent, index in self.agent_name_mapping.items():
             others = self._other_agents[agent]
-            self.observations[agent] = ObservationDict(
+            views[agent] = ObservationDict(
                 {
-                    'self': self._self_obs[:, index],
-                    'others': (lambda o=others: self._self_obs[:, o]),
-                    'tasks': (lambda i=index: jagged_rows_from_mask(self._task_obs, self.task_mask[:, i])),
-                    'tasks_padded': self._task_obs,
-                    'task_mask': self.task_mask[:, index],
+                    'self': self_obs[:, index],
+                    'others': (lambda o=others: self_obs[:, o]),
+                    'tasks': (lambda i=index: jagged_rows_from_mask(task_obs, task_mask[:, i])),
+                    'tasks_padded': task_obs,
+                    'task_mask': task_mask[:, index],
                 },
                 batch_size=[B],
                 device=self.device,
             )
+        return views
+
+    def update_observation_views(self) -> None:
+        self.observations = self._observation_views(self._observation_buffers())
         mapping = {a: (lambda i=i: jagged_indices_from_mask(self.task_mask[:, i])) for a, i in self.agent_name_mapping.items()}
         self.agent_action_mapping = LazyDict(dict(mapping))
         self.agent_observation_mapping = LazyDict(dict(mapping))

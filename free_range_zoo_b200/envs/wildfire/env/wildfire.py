@@ -299,7 +299,8 @@ class raw_env(BatchedAECEnv):
             static=tuple(f'init_{name}' for name in state) + (
                 'actions', 'cell_reward', 'cell_ignition', 'range_mask', 'cell_agents', 'control', 'field_uniforms',
                 'agent_uniforms'),
-            agents_with_tasks=True)
+            agents_with_tasks=True,
+            final=('self_obs', 'task_obs', 'action_mask', 'env_task_count', 'agent_task_count'))
 
     # ------------------------------------------------------------------------------------------ step
 
@@ -315,25 +316,27 @@ class raw_env(BatchedAECEnv):
         _lib.check(self._lib.frz_wildfire_refresh(ctypes.byref(self._params), ctypes.byref(self._io),
                                                   self.parallel_envs, self._stream()), 'frz_wildfire_refresh')
 
-    def _observation_download(self):
+    def _observation_download(self, buffers=None):
         """Host-side observation download (``gather_observations``): self observations and per-agent task counts whole,
         the live rows of the task observations and of every agent's action-mask row packed."""
-        dense = dict(self_obs=self._self_obs, agent_task_count=self._agent_task_count)
-        ragged = dict(task_obs=(self._task_obs, 1), action_mask=(self._action_mask, len(self.possible_agents)))
+        b = self._observation_buffers() if buffers is None else buffers
+        dense = dict(self_obs=b['self_obs'], agent_task_count=b['agent_task_count'])
+        ragged = dict(task_obs=(b['task_obs'], 1), action_mask=(b['action_mask'], len(self.possible_agents)))
         return dense, ragged
 
-    def _compact_schema(self):
+    def _compact_schema(self, buffers=None):
         """Compact download (utils/compact.py): live task rows and the action mask as bits; of ``self_obs`` only the
         suppressant -- y, x and power are the configuration's and are restored by ``unpack()``."""
+        b = self._observation_buffers() if buffers is None else buffers
         A, p = len(self.possible_agents), self._params
         bounds = compact_bounds(self.config)
         fill = torch.tensor([[float(p.agent_y[a]), float(p.agent_x[a]), p.agent_power[a], 0.0] for a in range(A)],
                             dtype=torch.float32)
         return compact.Schema(capacity=self.max_y * self.max_x, mask_groups=A, arrays=[
-            compact.rows('task_obs', self._task_obs, bound=bounds['task_obs']),
-            compact.mask('action_mask', self._action_mask, groups=A),
-            compact.dense('self_obs', self._self_obs, columns=(3, 1), fill=fill),
-            compact.dense('agent_task_count', self._agent_task_count, bound=bounds['agent_task_count']),
+            compact.rows('task_obs', b['task_obs'], bound=bounds['task_obs']),
+            compact.mask('action_mask', b['action_mask'], groups=A),
+            compact.dense('self_obs', b['self_obs'], columns=(3, 1), fill=fill),
+            compact.dense('agent_task_count', b['agent_task_count'], bound=bounds['agent_task_count']),
         ])
 
     def update_actions(self) -> None:
@@ -402,24 +405,30 @@ class raw_env(BatchedAECEnv):
         """Jagged int64 [B, #lit, 4] = (y, x, fires, intensity) like the reference (wildfire.py:699)."""
         return jagged_from_padded(self._task_obs, self.environment_task_count, torch.int64)
 
-    def update_observation_views(self) -> None:
+    def _observation_views(self, buffers) -> Dict[str, ObservationDict]:
         B = self.parallel_envs
-        tasks = LazyDict({'tasks': lambda: self.task_store})
-        self.observations = {}
+        self_obs, task_obs, counts = buffers['self_obs'], buffers['task_obs'], buffers['env_task_count']
+        action_mask = buffers['action_mask'][:, :, :self.max_y * self.max_x]
+        tasks = LazyDict({'tasks': lambda: jagged_from_padded(task_obs, counts, torch.int64)})
+        views = {}
         for agent, index in self.agent_name_mapping.items():
             others, columns = self._other_agents[agent], self._other_columns
-            self.observations[agent] = ObservationDict(
+            views[agent] = ObservationDict(
                 {
-                    'self': self._self_obs[:, index],
-                    'others': (lambda o=others, c=columns: self._self_obs[:, o][:, :, c]),
+                    'self': self_obs[:, index],
+                    'others': (lambda o=others, c=columns: self_obs[:, o][:, :, c]),
                     'tasks': (lambda: tasks['tasks']),
-                    'tasks_padded': self._task_obs,
-                    'task_count': self.environment_task_count,
-                    'action_mask': self.action_mask[:, index],
+                    'tasks_padded': task_obs,
+                    'task_count': counts,
+                    'action_mask': action_mask[:, index],
                 },
                 batch_size=[B],
                 device=self.device,
             )
+        return views
+
+    def update_observation_views(self) -> None:
+        self.observations = self._observation_views(self._observation_buffers())
         good = {a: (lambda i=i: jagged_indices_from_mask(self.action_mask[:, i] != 0))
                 for a, i in self.agent_name_mapping.items()}
         every = LazyDict({'all': lambda: jagged_indices_from_mask(

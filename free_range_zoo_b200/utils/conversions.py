@@ -83,3 +83,8 @@ class batched_aec_to_batched_parallel_wrapper:
     @property
     def finished(self) -> torch.Tensor:
         return self.aec_env.finished
+
+    @property
+    def final_observations(self) -> Dict[str, Any]:
+        """``BatchedAECEnv.final_observations``: the observations the episodes of the last step ended with."""
+        return self.aec_env.final_observations

@@ -46,6 +46,9 @@ class AutoresetRows(NamedTuple):
     overwritten: Tuple[str, ...]  # written for every environment by every step: kept as the finishing step wrote them
     static: Tuple[str, ...]  # not changed by a restart: init_* copies, inputs, configuration tables, the control block
     agents_with_tasks: bool  # whether the domain publishes FrzControl.agents_with_tasks (a refresh publishes 0 otherwise)
+    # the arrays the observations are built from (views and host downloads), all restored by a restart: what
+    # keep_final_observations copies aside before the restart overwrites them
+    final: Tuple[str, ...]
 
 
 class _DeviceBound:
@@ -103,6 +106,7 @@ class BatchedAECEnv(ABC):
         env_offset: int = 0,
         detach_outputs: bool = False,
         autoreset: bool = False,
+        keep_final_observations: bool = False,
         **kwargs,
     ):
         """
@@ -132,11 +136,19 @@ class BatchedAECEnv(ABC):
                 the finishing step produced; ``terminated`` / ``truncated`` / ``finished`` / ``terminations`` /
                 ``truncations`` read copies of the step's done flags ("the episode ended at the last step") and
                 ``episode_statistics`` gives each finished episode's return and length.  Restarted environments keep
-                drawing random numbers with the global step counter, as after ``reset_batches``.  The final observation
-                of a finished episode is not kept: the observations after the step are the restarted environment's.
-                Every full ``reset()`` snapshots the per-environment outputs of its refresh (observations, masks,
-                counts, rideshare's passenger table), which a restart copies back: about 2.8 KB per environment at
-                wildfire C4 (184 MB at 65 536 environments).  Not available with a ``log_directory``.
+                drawing random numbers with the global step counter, as after ``reset_batches``.  The observations
+                after the step are the restarted environment's; ``keep_final_observations`` keeps the ones the finished
+                episode ended with.  Every full ``reset()`` snapshots the per-environment outputs of its refresh
+                (observations, masks, counts, rideshare's passenger table), which a restart copies back: about 2.8 KB
+                per environment at wildfire C4 (184 MB at 65 536 environments).  Not available with a
+                ``log_directory``.
+            keep_final_observations: with ``autoreset`` only (``ValueError`` otherwise): before a restart overwrites
+                them, the restart copies the finished environments' observation arrays to a set of final-observation
+                buffers, in the same launch.  ``final_observations`` reads them on the device and
+                ``gather_observations(final=True)`` downloads them, e.g. to bootstrap a truncated episode from the value
+                of its last observation.  Costs one more copy of the observation arrays in device memory (as much again
+                as the snapshot at wildfire C4) and, on a step that finishes environments, one more pass over their
+                observation rows; nothing on a step where none finished.
         """
         device = torch.device(device)
         if device.type != 'cuda':
@@ -162,6 +174,10 @@ class BatchedAECEnv(ABC):
         if self.autoreset and log_directory is not None:
             raise ValueError('autoreset restarts environments on the device inside the step, which the logging tap does not '
                              'record; autoreset=True needs log_directory=None')
+        self.keep_final_observations = bool(keep_final_observations)
+        if self.keep_final_observations and not self.autoreset:
+            raise ValueError('keep_final_observations keeps what the autoreset overwrites: it needs autoreset=True '
+                             '(without it the observations of a finished environment stay until reset_batches)')
 
         if configuration is not None:
             self.config = configuration
@@ -254,6 +270,19 @@ class BatchedAECEnv(ABC):
         flags = self._autoreset_flags.view(torch.bool)
         return {'done': flags[0], 'terminated': flags[1], 'truncated': flags[2], 'return': self._episode_return,
                 'length': self._episode_length}
+
+    @property
+    def final_observations(self) -> Dict[str, ObservationDict]:
+        """The observations the episodes of the last step ended with (``keep_final_observations=True`` only):
+        ``{agent: ObservationDict}`` with the keys, shapes and dtypes of ``observations[agent]``, built over device
+        buffers that the next step overwrites where it finishes an environment.  Environment b's entry is the
+        observation its episode ended with wherever ``episode_statistics['done'][b]`` is set; elsewhere it holds an
+        earlier episode's or the last full ``reset()``'s observation, so select with ``done`` (e.g.
+        ``final_observations[agent]['self'][done]``).  ``reset_batches`` leaves them alone."""
+        if not self.keep_final_observations:
+            raise RuntimeError('final_observations are kept by the autoreset: construct the environment with '
+                               'autoreset=True, keep_final_observations=True')
+        return self._observation_views(self._final_buffers)
 
     @property
     def finished(self) -> torch.Tensor:
@@ -369,14 +398,22 @@ class BatchedAECEnv(ABC):
             self._reset_snapshot = {name: torch.empty_like(bound[name]) for name in rows.snapshot}
         for name, tensor in self._reset_snapshot.items():
             tensor.copy_(bound[name])
+        if self.keep_final_observations:  # (kept apart from _bound, which mirrors the domain's C buffer struct)
+            if getattr(self, '_final_buffers', None) is None:
+                self._final_buffers = {name: torch.empty_like(bound[name]) for name in rows.final}
+                self._final_counts = torch.zeros(B, dtype=torch.int32, device=self.device)
+            for name, tensor in self._final_buffers.items():  # well-formed before any episode has finished
+                tensor.copy_(bound[name])
+        keep = self._final_buffers if self.keep_final_observations else {}
         self._autoreset_flags.zero_()
-        pairs = ([(bound[dst], bound[src]) for dst, src in rows.init.items()] +
-                 [(bound[name], self._reset_snapshot[name]) for name in rows.snapshot] +
-                 [(bound[name], None) for name in rows.zero])
+        pairs = ([(name, bound[src]) for name, src in rows.init.items()] +
+                 [(name, self._reset_snapshot[name]) for name in rows.snapshot] +
+                 [(name, None) for name in rows.zero])
         table = (_lib.AutoresetRow * len(pairs))()
-        for at, (dst, src) in enumerate(pairs):
+        for at, (name, src) in enumerate(pairs):
+            dst = bound[name]
             assert dst.shape[0] == B and dst.is_contiguous() and (src is None or src.shape == dst.shape)
-            table[at].dst, table[at].src = dst.data_ptr(), _lib.pointer(src)
+            table[at].dst, table[at].src, table[at].keep = dst.data_ptr(), _lib.pointer(src), _lib.pointer(keep.get(name))
             table[at].bytes = dst.numel() * dst.element_size() // B
         block = _lib.Autoreset()
         block.terminated, block.truncated = self._terminated.data_ptr(), self._truncated.data_ptr()
@@ -490,18 +527,49 @@ class BatchedAECEnv(ABC):
 
     # ------------------------------------------------------------------------------------------ observations on the host
 
-    def _observation_download(self) -> Tuple[Dict[str, torch.Tensor], Dict[str, Tuple[torch.Tensor, int]]]:
-        """What a policy on the host reads after a step: ``(dense, ragged)``.  ``dense`` arrays leave the device whole;
-        ``ragged`` maps a name to ``(padded array [B, groups, capacity, ...] or [B, capacity, ...], groups)`` of which
-        only the first ``environment_task_count[b]`` rows per environment (and row block) are live.  Domain hook."""
+    def _observation_buffers(self) -> Dict[str, torch.Tensor]:
+        """The live arrays the observations are built from, by ``_bound`` name (``_autoreset_rows().final``); the
+        final-observation buffers have the same names."""
+        buffers = self.__dict__.get('_live_observation_buffers')
+        if buffers is None:  # (the tensors live as long as the environment; rebinding keeps them)
+            buffers = self._live_observation_buffers = {name: self._bound[name] for name in self._autoreset_rows().final}
+        return buffers
+
+    def _observation_views(self, buffers: Dict[str, torch.Tensor]) -> Dict[str, ObservationDict]:
+        """``{agent: ObservationDict}`` as views of ``buffers`` (live or final, see ``_observation_buffers``).  Domain
+        hook."""
         raise NotImplementedError
 
-    def _gather_state(self):
-        state = getattr(self, '_gather', None)
+    def _observation_download(self, buffers: Optional[Dict[str, torch.Tensor]] = None
+                              ) -> Tuple[Dict[str, torch.Tensor], Dict[str, Tuple[torch.Tensor, int]]]:
+        """What a policy on the host reads after a step, from ``buffers`` (None = the live ones): ``(dense, ragged)``.
+        ``dense`` arrays leave the device whole; ``ragged`` maps a name to ``(padded array [B, groups, capacity, ...] or
+        [B, capacity, ...], groups)`` of which only the first ``counts[b]`` rows per environment (and row block) are
+        live.  Domain hook."""
+        raise NotImplementedError
+
+    def _download_counts(self, final: bool) -> torch.Tensor:
+        """Live rows per environment of a download: the task counts, or for the final observations the final counts
+        of the environments the last step finished and 0 elsewhere (computed on the current stream)."""
+        if not final:
+            return self.environment_task_count
+        done = self._autoreset_flags[0]  # uint8 0 / 1
+        torch.mul(self._final_buffers['env_task_count'], done, out=self._final_counts)
+        return self._final_counts
+
+    def _download_buffers(self, final: bool) -> Dict[str, torch.Tensor]:
+        if final and not self.keep_final_observations:
+            raise RuntimeError('final observations are kept by the autoreset: construct the environment with '
+                               'autoreset=True, keep_final_observations=True')
+        return self._final_buffers if final else self._observation_buffers()
+
+    def _gather_state(self, final: bool = False):
+        attribute = '_gather_final' if final else '_gather'
+        state = getattr(self, attribute, None)
         if state is not None:
             return state
         B, dev = self.parallel_envs, self.device
-        dense, ragged = self._observation_download()
+        dense, ragged = self._observation_download(self._download_buffers(final))
         arrays = (_lib.GatherArray * max(1, len(ragged)))()
         packed, layout = {}, {}
         for at, (name, (tensor, groups)) in enumerate(ragged.items()):
@@ -513,7 +581,7 @@ class BatchedAECEnv(ABC):
             arrays[at].row_bytes, arrays[at].capacity, arrays[at].groups = row_bytes, capacity, groups
             layout[name] = (groups, row_shape, row_bytes // tensor.element_size())
         state = dict(
-            dense=dense, ragged=ragged, arrays=arrays, packed=packed, layout=layout,
+            final=final, dense=dense, ragged=ragged, arrays=arrays, packed=packed, layout=layout,
             offsets=torch.zeros(B + 1, dtype=torch.int32, device=dev),
             scratch=torch.zeros((B + 1023) // 1024 + 1, dtype=torch.int32, device=dev),
             host_counts=torch.zeros(B, dtype=torch.int32).pin_memory(),
@@ -521,16 +589,17 @@ class BatchedAECEnv(ABC):
             host_dense={name: torch.empty(tensor.shape, dtype=tensor.dtype).pin_memory() for name, tensor in dense.items()},
             host_packed={name: torch.empty(tensor.numel(), dtype=tensor.dtype).pin_memory() for name, tensor in packed.items()},
         )
-        self._gather = state
+        setattr(self, attribute, state)
         return state
 
     def _enqueue_gather(self, state) -> None:
         """Compaction kernels + the downloads whose size is known up front (counts, offsets, dense arrays), on the
         current stream of the device."""
-        _lib.check(self._lib.frz_gather_live_rows(self.environment_task_count.data_ptr(), self.parallel_envs,
+        counts = self._download_counts(state['final'])
+        _lib.check(self._lib.frz_gather_live_rows(counts.data_ptr(), self.parallel_envs,
                                                   state['offsets'].data_ptr(), state['scratch'].data_ptr(), state['arrays'],
                                                   len(state['ragged']), self._stream()), 'frz_gather_live_rows')
-        state['host_counts'].copy_(self.environment_task_count, non_blocking=True)
+        state['host_counts'].copy_(counts, non_blocking=True)
         state['host_offsets'].copy_(state['offsets'], non_blocking=True)
         for name, tensor in state['dense'].items():
             state['host_dense'][name].copy_(tensor, non_blocking=True)
@@ -557,27 +626,31 @@ class BatchedAECEnv(ABC):
         out['bytes'] = moved
         return out
 
-    def _compact_schema(self) -> compact.Schema:
-        """The domain's compact observation format (utils/compact.py): which array is narrowed to which type, from
-        bounds the configuration guarantees.  Domain hook."""
+    def _compact_schema(self, buffers: Optional[Dict[str, torch.Tensor]] = None) -> compact.Schema:
+        """The domain's compact observation format (utils/compact.py) over ``buffers`` (None = the live ones): which
+        array is narrowed to which type, from bounds the configuration guarantees.  Domain hook."""
         raise NotImplementedError
 
-    def _compact_download(self) -> compact.CompactDownload:
-        download = getattr(self, '_compact', None)
+    def _compact_download(self, final: bool = False) -> compact.CompactDownload:
+        attribute = '_compact_final' if final else '_compact'
+        download = getattr(self, attribute, None)
         if download is None or download.key != self.max_steps:  # (rideshare bounds depend on the horizon)
-            download = compact.CompactDownload(self._compact_schema(), self.environment_task_count, key=self.max_steps)
-            self._compact = download
+            schema = self._compact_schema(self._download_buffers(final))
+            counts = self._final_counts if final else self.environment_task_count
+            download = compact.CompactDownload(schema, counts, key=self.max_steps)
+            setattr(self, attribute, download)
         return download
 
-    def _enqueue_compact(self) -> compact.CompactDownload:
+    def _enqueue_compact(self, final: bool = False) -> compact.CompactDownload:
         """The compact download of the current state (frz_observe_compact), on the current stream of the device."""
-        download = self._compact_download()
+        download = self._compact_download(final)
+        self._download_counts(final)
         _lib.check(self._lib.frz_observe_compact(ctypes.byref(download.block), self.parallel_envs, self._stream()),
                    'frz_observe_compact')
         return download
 
     @torch.no_grad()
-    def gather_observations(self, compact: bool = False) -> Dict[str, Any]:
+    def gather_observations(self, compact: bool = False, final: bool = False) -> Dict[str, Any]:
         """The observations of the current state in page-locked HOST memory, packed like the reference's jagged nested
         tensors (a value buffer + offsets; wildfire.py:669-717, rideshare.py:398-467): ``counts`` int32 [B] live tasks
         per environment, ``offsets`` int32 [B + 1] their exclusive prefix sum, the dense arrays (``self_obs``,
@@ -589,13 +662,18 @@ class BatchedAECEnv(ABC):
 
         ``compact=True`` returns the same observations in the compact format instead (a ``CompactObservations``,
         utils/compact.py: narrow integers, bit masks, no configuration constants; ``.unpack()`` gives this dict), encoded
-        on the device and stored straight into page-locked host buffers: one synchronisation, fewer bytes."""
+        on the device and stored straight into page-locked host buffers: one synchronisation, fewer bytes.
+
+        ``final=True`` (``keep_final_observations=True`` only) downloads ``final_observations`` instead, in either
+        format: ``counts`` is environment b's final task count where ``episode_statistics['done'][b]`` is set and 0
+        elsewhere, so only the finished environments' rows cross the link; the dense arrays come whole and are defined
+        where ``done`` is set.  Its host buffers are separate from those of the live download."""
         with torch.cuda.device(self.device):
             if compact:
-                download = self._enqueue_compact()
+                download = self._enqueue_compact(final)
                 torch.cuda.current_stream(self.device).synchronize()
                 return download.result()
-            state = self._gather_state()
+            state = self._gather_state(final)
             self._enqueue_gather(state)
             torch.cuda.current_stream(self.device).synchronize()
             return self._finish_gather(state)
@@ -799,6 +877,8 @@ class BatchedAECEnv(ABC):
         saved = {name: tensor.clone() for name, tensor in self._bound.items()
                  if tensor is not None and not name.startswith('init_')}
         autoreset = [self._autoreset_flags, self._episode_return, self._episode_length] if self.autoreset else []
+        if self.keep_final_observations:
+            autoreset += list(self._final_buffers.values())
         saved_autoreset = [tensor.clone() for tensor in autoreset]
         side = torch.cuda.Stream(self.device)
         side.wait_stream(torch.cuda.current_stream(self.device))

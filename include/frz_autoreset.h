@@ -13,6 +13,11 @@
  * refresh of the restored state would write); AEC fields such as the done flags and the cumulative rewards are zeroed.
  * The library knows row descriptors only, never domains.
  *
+ * A learner that bootstraps a truncated episode from the value of its last observation needs that observation after
+ * the restart has overwritten it.  A row with a `keep` array has its current bytes copied there before it is restored:
+ * the lane that restores a word loads the old word first, so the copy costs no launch and no ordering, and moves the
+ * row's bytes once more for finished environments only.
+ *
  * One call, for B = parallel_envs environments:
  *  1. scan (one pass over B): done[b] = terminated[b] | truncated[b]; step_terminated / step_truncated / done receive
  *     copies of the flags the step produced (the live flags are zeroed by the restart); for finished environments
@@ -22,7 +27,8 @@
  *     is finished) and agents_with_tasks = OR over agents with a task, from agent_task_count of the environments that
  *     did not finish and reset_agent_task_count of those that did.  The step counter is left alone: restarted
  *     environments keep drawing with the global step counter, as after frz_<domain>_reset.
- *  2. restore: every row of every listed environment is copied from src (or zeroed).
+ *  2. restore: every row of every listed environment is copied from src (or zeroed), after its current value has
+ *     been copied to keep where the row has one.
  * No host read: capturable.
  */
 #ifndef FRZ_AUTORESET_H_
@@ -36,11 +42,14 @@ extern "C" {
 
 #define FRZ_AUTORESET_MAX_ROWS 32
 
-/* One per-environment array restored by a restart: dst[b] <- src[b] (or zeros), `bytes` bytes per environment. */
+/* One per-environment array restored by a restart: keep[b] <- dst[b] (if keep), then dst[b] <- src[b] (or zeros),
+   `bytes` bytes per environment. */
 typedef struct {
   void* dst;              /* device [B, bytes] */
   const void* src;        /* device [B, bytes], or NULL: zero the row */
   int64_t bytes;          /* > 0 */
+  void* keep;             /* device [B, bytes], or NULL: before a finished environment's row is restored, its current
+                             bytes are copied to keep[b] */
 } FrzAutoresetRow;
 
 typedef struct {

@@ -2,10 +2,11 @@
 
     python profiles/time_autoreset.py [--out r4_autoreset.json] [--windows 5] [--graph-steps 10]
 
-Three variants of one engine over whole episodes of ``max_steps`` = 100 steps (the horizon of every named workload),
+Four variants of one engine over whole episodes of ``max_steps`` = 100 steps (the horizon of every named workload),
 actions sampled on the device:
   off       ``autoreset=False``: ``capture_graph(sample=True, steps=K)`` replays
   on        ``autoreset=True``: the same replays, the autoreset launches captured after every step
+  final     ``autoreset=True, keep_final_observations=True``: as ``on``, the restore also keeps the final observations
   explicit  ``autoreset=False`` with ``reset_batches(finished)`` after every step (eager: the index list needs the host)
 Each window resets the engine (untimed), then times one episode with CUDA events; windows alternate between the
 variants.  env-steps/s = B x max_steps / episode time (the nominal step count: after every environment of an ``off``
@@ -13,7 +14,8 @@ batch has terminated, its remaining steps are no-ops).
 
 The autoreset launches alone, inside a graph of 20 back-to-back calls: on a step where no environment finished, and
 where every environment is truncated (the graph sets every truncated flag before each call; the same graph without the
-autoreset is subtracted).  The working sets are smaller than L2 at C4 and larger at the 524 288-environment workloads.
+autoreset is subtracted), for ``on`` and for ``final``.  The working sets are smaller than L2 at C4 and larger at the
+524 288-environment workloads.
 """
 import argparse
 import importlib
@@ -44,13 +46,14 @@ def gpu_description():
     return info
 
 
-def make(domain, preset, kwargs, B, autoreset):
+def make(domain, preset, kwargs, B, autoreset, keep=False):
     import torch
 
     from free_range_zoo_b200 import presets
     module = importlib.import_module(f'free_range_zoo_b200.envs.{domain}_v0')
     env = module.parallel_env(parallel_envs=B, max_steps=MAX_STEPS, configuration=getattr(presets, preset)(),
-                              device=torch.device('cuda:0'), autoreset=autoreset, **kwargs)
+                              device=torch.device('cuda:0'), autoreset=autoreset,
+                              keep_final_observations=keep, **kwargs)
     return env.unwrapped
 
 
@@ -111,8 +114,8 @@ def autoreset_launch_us(torch, raw, every_truncated):
 def measure(name, domain, preset, kwargs, B, windows, graph_steps):
     import torch
     engines = {'off': make(domain, preset, kwargs, B, False), 'on': make(domain, preset, kwargs, B, True),
-               'explicit': make(domain, preset, kwargs, B, False)}
-    for variant in ('off', 'on'):
+               'final': make(domain, preset, kwargs, B, True, keep=True), 'explicit': make(domain, preset, kwargs, B, False)}
+    for variant in ('off', 'on', 'final'):
         engines[variant].reset(seed=SEED)
         engines[variant].capture_graph(sample=True, sampler_seed=SAMPLER, steps=graph_steps)
     for variant, raw in engines.items():  # warm-up episode
@@ -123,16 +126,20 @@ def measure(name, domain, preset, kwargs, B, windows, graph_steps):
             times[variant].append(episode(torch, raw, variant, graph_steps))
     rate = {variant: [B * MAX_STEPS / (ms * 1e-3) for ms in values] for variant, values in times.items()}
     median = {variant: statistics.median(values) for variant, values in times.items()}
-    on = engines['on']
+    on, final = engines['on'], engines['final']
     row = dict(workload=name, parallel_envs=B, max_steps=MAX_STEPS, graph_steps=graph_steps, windows=windows,
                episode_ms=times, env_steps_per_s=rate,
                env_steps_per_s_median={variant: B * MAX_STEPS / (ms * 1e-3) for variant, ms in median.items()},
                autoreset_overhead_pct=100.0 * (median['on'] / median['off'] - 1.0),
+               final_overhead_pct=100.0 * (median['final'] / median['on'] - 1.0),
                explicit_step_ms=median['explicit'] / MAX_STEPS, off_step_ms=median['off'] / MAX_STEPS,
                autoreset_us_nothing_finished=autoreset_launch_us(torch, on, False),
                autoreset_us_every_env_truncated=autoreset_launch_us(torch, on, True),
-               snapshot_bytes_per_env=sum(t.numel() * t.element_size() for t in on._reset_snapshot.values()) // B)
-    del engines, on
+               final_us_nothing_finished=autoreset_launch_us(torch, final, False),
+               final_us_every_env_truncated=autoreset_launch_us(torch, final, True),
+               snapshot_bytes_per_env=sum(t.numel() * t.element_size() for t in on._reset_snapshot.values()) // B,
+               final_bytes_per_env=sum(t.numel() * t.element_size() for t in final._final_buffers.values()) // B)
+    del engines, on, final
     torch.cuda.empty_cache()
     return row
 
