@@ -28,6 +28,8 @@ FAULT_NAMES = {
     0x2: 'cybersecurity attack / movement target outside [0, num_nodes)',
     0x4: 'a non-present cybersecurity agent acted while show_bad_actions=False',
     0x8: 'rideshare passenger table overflow',
+    0x10: 'policy logits are NaN or +inf in a legal slot, or -inf in every legal slot (decoded as the noop)',
+    0x20: 'a policy slot is out of range or not legal (decoded as the noop)',
 }
 
 
@@ -178,6 +180,16 @@ class Autoreset(C.Structure):
                                          ('num_agents', C.c_int32)]
 
 
+class PolicyActions(C.Structure):
+    """FrzPolicyActions (include/frz_policy.h): mode, logits and outputs of one policy-actions launch."""
+    _fields_ = [('mode', C.c_int32), ('logits_type', C.c_int32), ('logits', C.c_void_p), ('slots', C.c_int32),
+                ('row_stride', C.c_int32), ('slot', C.c_void_p), ('log_prob', C.c_void_p), ('legal', C.c_void_p),
+                ('sampler_seed', C.c_uint64)]
+
+
+POLICY_SAMPLE, POLICY_DECODE, POLICY_LEGAL = 0, 1, 2
+LOGITS_F32, LOGITS_BF16 = 0, 1
+
 OBS_DENSE, OBS_ROWS, OBS_MASK_BITS = 0, 1, 2
 OBS_I32, OBS_I16, OBS_I8, OBS_U8, OBS_F32 = 0, 1, 2, 3, 4
 HOST_ACTIONS_I32, HOST_ACTIONS_I16, HOST_ACTIONS_I8 = 0, 1, 2
@@ -226,6 +238,11 @@ def library() -> C.CDLL:
                                          C.c_void_p]
     lib.frz_observe_compact.argtypes = [C.POINTER(ObsDownload), C.c_int32, C.c_void_p]
     lib.frz_autoreset.argtypes = [C.POINTER(Autoreset), C.c_int32, C.c_void_p]
+    for name, params, buffers in (('frz_wildfire_policy_actions', WildfireParams, WildfireBuffers),
+                                  ('frz_cyber_policy_actions', CyberParams, CyberBuffers),
+                                  ('frz_rideshare_policy_actions', RideshareParams, RideshareBuffers)):
+        getattr(lib, name).argtypes = [C.POINTER(params), C.POINTER(buffers), C.c_int32, C.POINTER(PolicyActions),
+                                       C.c_void_p]
     if lib.frz_version() != ABI_VERSION:
         raise RuntimeError(f'libfrz.so ABI version {lib.frz_version()} != {ABI_VERSION}; rebuild the library')
     lib.frz_control_restore.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p]

@@ -309,6 +309,15 @@ class raw_env(BatchedAECEnv):
                    'frz_cyber_sample_actions')
         return self._actions
 
+    @property
+    def action_slots(self) -> int:
+        """N + 3 for every agent: slot t < N attacks / moves to node t, then noop, patch and monitor (the last two are
+        never legal for attackers)."""
+        return int(self._params.num_nodes) + 3
+
+    def _policy_entry(self):
+        return self._lib.frz_cyber_policy_actions
+
     # ------------------------------------------------------------------------------------------ views
 
     @property

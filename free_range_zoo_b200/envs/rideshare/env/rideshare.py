@@ -257,6 +257,14 @@ class raw_env(BatchedAECEnv):
                                                           self._stream()), 'frz_rideshare_sample_actions')
         return self._actions
 
+    @property
+    def action_slots(self) -> int:
+        """K + 1: slot t < K acts on passenger-table row t with the id its state requires, slot K is the noop."""
+        return int(self._params.capacity) + 1
+
+    def _policy_entry(self):
+        return self._lib.frz_rideshare_policy_actions
+
     # ------------------------------------------------------------------------------------------ logging tap
 
     def _log_snapshot(self) -> Dict[str, torch.Tensor]:

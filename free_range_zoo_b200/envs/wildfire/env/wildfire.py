@@ -362,6 +362,14 @@ class raw_env(BatchedAECEnv):
                                                          self._stream()), 'frz_wildfire_sample_actions')
         return self._actions
 
+    @property
+    def action_slots(self) -> int:
+        """H*W + 1: slot t < H*W acts on env-local task t (row t of ``tasks_padded``), slot H*W is the noop."""
+        return int(self._params.height) * int(self._params.width) + 1
+
+    def _policy_entry(self):
+        return self._lib.frz_wildfire_policy_actions
+
     # ------------------------------------------------------------------------------------------ logging tap
 
     def _log_snapshot(self) -> Dict[str, torch.Tensor]:

@@ -915,3 +915,99 @@ class BatchedAECEnv(ABC):
         """Uniform random legal actions for every agent, generated on the device into the staged action table
         (the caller side of the path: replaces ``action_space(agent).sample_nested()`` per agent per step)."""
         raise NotImplementedError
+
+    # ------------------------------------------------------------------------------------------ policy actions
+
+    @property
+    def action_slots(self) -> int:
+        """C: the fixed number of action slots per agent a policy scores (include/frz_policy.h) -- wildfire H*W + 1
+        (slot t acts on env-local task t, the last is the noop), rideshare K + 1 (table row t, then the noop),
+        cybersecurity N + 3 (node t, then noop, patch, monitor).  The legal slots of (environment, agent) are, in slot
+        order, the choices of ``action_space(agent)`` for that environment.  Domain hook."""
+        raise NotImplementedError
+
+    def _policy_entry(self):
+        """The domain's ``frz_<domain>_policy_actions`` entry point."""
+        raise NotImplementedError
+
+    def _policy_buffers(self) -> Dict[str, torch.Tensor]:
+        """Env-owned outputs of the policy launches, allocated by the first call (later calls allocate nothing)."""
+        buffers = self.__dict__.get('_policy')
+        if buffers is None:
+            B, A, dev = self.parallel_envs, len(self.possible_agents), self.device
+            buffers = self._policy = dict(slots=torch.zeros((B, A), dtype=torch.int32, device=dev),
+                                          log_prob=torch.zeros((B, A), dtype=torch.float32, device=dev),
+                                          legal=torch.zeros((B, A, self.action_slots), dtype=torch.bool, device=dev))
+        return buffers
+
+    def _check_policy_tensor(self, tensor: torch.Tensor, what: str, dtypes, slots: bool = True) -> None:
+        B, A = self.parallel_envs, len(self.possible_agents)
+        shape = (B, A, self.action_slots) if slots else (B, A)
+        if not isinstance(tensor, torch.Tensor) or tensor.device != self.device or tensor.dtype not in dtypes \
+                or tuple(tensor.shape) != shape:
+            raise ValueError(f'{what} must be a {" / ".join(str(d) for d in dtypes)} tensor of shape {shape} on '
+                             f'{self.device}')
+
+    def _policy_launch(self, mode: int, logits: Optional[torch.Tensor] = None, legal: Optional[torch.Tensor] = None,
+                       sampler_seed: int = 0) -> None:
+        buffers = self._policy_buffers()
+        block = _lib.PolicyActions()
+        block.mode, block.slots = mode, self.action_slots
+        block.slot, block.log_prob = buffers['slots'].data_ptr(), buffers['log_prob'].data_ptr()
+        block.legal = _lib.pointer(legal)
+        block.sampler_seed = int(sampler_seed) & 0xFFFFFFFFFFFFFFFF
+        if logits is not None:
+            block.logits, block.row_stride = logits.data_ptr(), logits.stride(1)
+            block.logits_type = _lib.LOGITS_BF16 if logits.dtype == torch.bfloat16 else _lib.LOGITS_F32
+        _lib.check(self._policy_entry()(ctypes.byref(self._params), ctypes.byref(self._io), self.parallel_envs,
+                                        ctypes.byref(block), self._stream()), 'policy_actions')
+
+    def legal_actions(self, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """bool [B, A, C] on the device: slot t of (environment, agent) is legal (``action_slots``).  Written into
+        ``out`` (bool or uint8, contiguous) when given, else into an env-owned buffer the next call overwrites."""
+        if out is None:
+            out = self._policy_buffers()['legal']
+        else:
+            self._check_policy_tensor(out, 'out', (torch.bool, torch.uint8))
+            if not out.is_contiguous():
+                raise ValueError('out must be contiguous')
+        self._policy_launch(_lib.POLICY_LEGAL, legal=out)
+        return out
+
+    def sample_actions_from_logits(self, logits: torch.Tensor, sampler_seed: int = 2026,
+                                   legal_out: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Sample every agent's action from ``logits`` (f32 or bf16 [B, A, C] on the device, C = ``action_slots``; rows
+        may be a view with a larger stride, e.g. ``wide[..., :C]``) restricted to the legal slots, and stage it for
+        ``step_all(None)`` / the Parallel ``step``.  One launch, no host read: capturable in a CUDA graph.
+
+        Returns ``(slots, log_prob)``: int32 [B, A] chosen slots and f32 [B, A] their log-probability under the masked
+        softmax, env-owned buffers overwritten by the next call.  ``legal_out`` (bool / uint8 [B, A, C], contiguous)
+        receives the legal mask in the same launch, e.g. for a learner that recomputes log-probabilities with gradients.
+        The random draw of (environment, agent) is the one ``sample_actions(sampler_seed)`` makes, so equal logits
+        stage exactly what ``sample_actions`` stages.  NaN / +inf in a legal slot, or -inf in all of them, records a
+        fault (``check_errors``) and stages the noop."""
+        self._check_policy_tensor(logits, 'logits', (torch.float32, torch.bfloat16))
+        if logits.stride(2) != 1 or logits.stride(0) != logits.stride(1) * logits.shape[1]:
+            raise ValueError('logits rows must be evenly spaced with unit stride along the slots '
+                             '(a contiguous tensor, or a [..., :C] view of one)')
+        if legal_out is not None:
+            self._check_policy_tensor(legal_out, 'legal_out', (torch.bool, torch.uint8))
+            if not legal_out.is_contiguous():
+                raise ValueError('legal_out must be contiguous')
+        self._policy_launch(_lib.POLICY_SAMPLE, logits=logits, legal=legal_out, sampler_seed=sampler_seed)
+        buffers = self._policy_buffers()
+        return buffers['slots'], buffers['log_prob']
+
+    def actions_from_slots(self, slots: torch.Tensor) -> torch.Tensor:
+        """Stage the actions of chosen slots (int [B, A], on the device or the host), e.g. a greedy
+        ``logits.masked_fill(~legal, -inf).argmax(-1)`` or a CPU policy's choices.  An out-of-range or illegal slot
+        records a fault (``check_errors``) and stages the noop.  Returns the staged [B, A, 2] action table."""
+        shape = (self.parallel_envs, len(self.possible_agents))
+        if not isinstance(slots, torch.Tensor) or tuple(slots.shape) != shape or slots.is_floating_point() \
+                or slots.is_complex() or slots.dtype == torch.bool:
+            raise ValueError(f'slots must be an integer tensor of shape {shape}')
+        buffers = self._policy_buffers()
+        if slots.data_ptr() != buffers['slots'].data_ptr():
+            buffers['slots'].copy_(slots, non_blocking=True)
+        self._policy_launch(_lib.POLICY_DECODE)
+        return self._actions
