@@ -190,6 +190,25 @@ class PolicyActions(C.Structure):
 POLICY_SAMPLE, POLICY_DECODE, POLICY_LEGAL = 0, 1, 2
 LOGITS_F32, LOGITS_BF16 = 0, 1
 
+INPUTS_MAX_COLUMNS = 8
+
+
+class InputColumns(C.Structure):
+    """FrzInputColumns (include/frz_inputs.h): per-column scale / offset of one source array of the policy inputs."""
+    _fields_ = [('scale', C.c_float * INPUTS_MAX_COLUMNS), ('offset', C.c_int32 * INPUTS_MAX_COLUMNS),
+                ('columns', C.c_int32), ('observed', C.c_uint32), ('pad_is_none', C.c_uint32), ('reserved', C.c_int32)]
+
+
+class PolicyInputs(C.Structure):
+    """FrzPolicyInputs (include/frz_inputs.h): outputs, widths and column tables of one policy-inputs launch."""
+    _fields_ = [('agent', C.c_void_p), ('tasks', C.c_void_p), ('output_type', C.c_int32), ('agent_width', C.c_int32),
+                ('task_width', C.c_int32), ('views', C.c_int32), ('task_rows', C.c_int32), ('flags', C.c_uint32),
+                ('self_columns', InputColumns * 2), ('task_columns', InputColumns)]
+
+
+INPUTS_F32, INPUTS_BF16 = 0, 1
+INPUTS_PARTIALLY_OBSERVABLE = 0x1
+
 OBS_DENSE, OBS_ROWS, OBS_MASK_BITS = 0, 1, 2
 OBS_I32, OBS_I16, OBS_I8, OBS_U8, OBS_F32 = 0, 1, 2, 3, 4
 HOST_ACTIONS_I32, HOST_ACTIONS_I16, HOST_ACTIONS_I8 = 0, 1, 2
@@ -242,6 +261,11 @@ def library() -> C.CDLL:
                                   ('frz_cyber_policy_actions', CyberParams, CyberBuffers),
                                   ('frz_rideshare_policy_actions', RideshareParams, RideshareBuffers)):
         getattr(lib, name).argtypes = [C.POINTER(params), C.POINTER(buffers), C.c_int32, C.POINTER(PolicyActions),
+                                       C.c_void_p]
+    for name, params, buffers in (('frz_wildfire_policy_inputs', WildfireParams, WildfireBuffers),
+                                  ('frz_cyber_policy_inputs', CyberParams, CyberBuffers),
+                                  ('frz_rideshare_policy_inputs', RideshareParams, RideshareBuffers)):
+        getattr(lib, name).argtypes = [C.POINTER(params), C.POINTER(buffers), C.c_int32, C.POINTER(PolicyInputs),
                                        C.c_void_p]
     if lib.frz_version() != ABI_VERSION:
         raise RuntimeError(f'libfrz.so ABI version {lib.frz_version()} != {ABI_VERSION}; rebuild the library')

@@ -19,7 +19,8 @@ from free_range_zoo_b200.envs.cybersecurity.env.structures.state import Cybersec
 from free_range_zoo_b200.utils.containers import LazyDict, ObservationDict, jagged_indices_from_mask
 from free_range_zoo_b200.utils.conversions import batched_aec_to_batched_parallel
 from free_range_zoo_b200.utils import compact
-from free_range_zoo_b200.utils.env import AutoresetRows, BatchedAECEnv
+from free_range_zoo_b200.utils.env import (AutoresetRows, BatchedAECEnv, InputKind, PolicyInputLayout,
+                                           PolicyInputSchema, input_column)
 from free_range_zoo_b200.utils.spaces import BatchedActionSpace, Space
 
 
@@ -101,9 +102,12 @@ def flatten_configuration(config, max_steps, show_bad_actions: bool, env_offset:
 def compact_bounds(params) -> Dict[str, int]:
     """Largest |value| of the integer observations, from the configuration (utils/compact.py picks the types): task
     rows hold (state, criticality), task counts at most every subnetwork."""
-    N = int(params.num_nodes)
-    criticality = max(abs(int(params.criticality[n])) for n in range(N))
-    return dict(task_obs=max(int(params.num_states) - 1, criticality), agent_task_count=N)
+    return dict(task_obs=max(int(params.num_states) - 1, max_criticality(params)), agent_task_count=int(params.num_nodes))
+
+
+def max_criticality(params) -> int:
+    """Largest |criticality| of the configuration's subnetworks."""
+    return max(abs(int(params.criticality[n])) for n in range(int(params.num_nodes)))
 
 
 class raw_env(BatchedAECEnv):
@@ -317,6 +321,32 @@ class raw_env(BatchedAECEnv):
 
     def _policy_entry(self):
         return self._lib.frz_cyber_policy_actions
+
+    def _policy_input_layout(self) -> PolicyInputLayout:
+        """Attackers (threat, presence), defenders (mitigation, presence, location), each with the observed columns of
+        the other agents of its kind; one view of the (state, criticality) rows per agent."""
+        p = self._params
+        power, presence = self.observe_other_power, self.observe_other_presence
+        attacker = tuple(c for c, on in enumerate((power, presence)) if on)
+        defender = tuple(c for c, on in enumerate((power, presence, self.observe_other_location)) if on)
+        return PolicyInputLayout(
+            kinds=(InputKind(int(p.num_attackers), 2, attacker), InputKind(int(p.num_defenders), 3, defender)),
+            task_rows=int(p.num_nodes), views=int(p.num_attackers) + int(p.num_defenders), task_columns=(False, False),
+            flags=_lib.INPUTS_PARTIALLY_OBSERVABLE if self.partially_observable else 0)
+
+    def _policy_input_schema(self) -> PolicyInputSchema:
+        """``1 / high`` of the configuration's observation bounds; the defender location maps home (-1) to 0 and node
+        n to (n + 1) / N; criticality, which ``observation_space`` leaves unbounded, is scaled by the largest
+        |criticality|."""
+        config = self.config
+        attacker = tuple(input_column(h) for h in config.attacker_observation_bounds)
+        mitigation, presence, location = config.defender_observation_bounds
+        defender = (input_column(mitigation), input_column(presence), input_column(location, none=True))
+        tasks = (input_column(config.network_observation_bounds[0]), input_column(max_criticality(self._params)))
+        return PolicyInputSchema(self._policy_input_layout(), self_columns=(attacker, defender), task_columns=tasks)
+
+    def _inputs_entry(self):
+        return self._lib.frz_cyber_policy_inputs
 
     # ------------------------------------------------------------------------------------------ views
 

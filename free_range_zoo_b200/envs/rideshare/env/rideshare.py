@@ -19,7 +19,8 @@ from free_range_zoo_b200.utils.containers import (LazyDict, ObservationDict, jag
                                                   jagged_rows_from_mask)
 from free_range_zoo_b200.utils.conversions import batched_aec_to_batched_parallel
 from free_range_zoo_b200.utils import compact
-from free_range_zoo_b200.utils.env import AutoresetRows, BatchedAECEnv
+from free_range_zoo_b200.utils.env import (AutoresetRows, BatchedAECEnv, InputKind, PolicyInputLayout,
+                                           PolicyInputSchema, input_column)
 from free_range_zoo_b200.utils.spaces import BatchedActionSpace, Space
 
 
@@ -264,6 +265,26 @@ class raw_env(BatchedAECEnv):
 
     def _policy_entry(self):
         return self._lib.frz_rideshare_policy_actions
+
+    # the task columns accepted_by / riding_by hold a driver index or FRZ_PAD for nobody
+    _NONE_TASK_COLUMNS = (False, ) * 4 + (True, True) + (False, ) * 2
+
+    def _policy_input_layout(self) -> PolicyInputLayout:
+        """Self (y, x, #accepted, #riding), the same four of every other driver; every passenger row, one view."""
+        p = self._params
+        return PolicyInputLayout(kinds=(InputKind(int(p.num_agents), 4, (0, 1, 2, 3)), ), task_rows=int(p.capacity),
+                                 views=1, task_columns=self._NONE_TASK_COLUMNS)
+
+    def _policy_input_schema(self) -> PolicyInputSchema:
+        """``1 / high`` of ``agent_observation_bounds`` and ``passenger_observation_bounds``; accepted_by / riding_by
+        map nobody to 0 and driver i to (i + 1) / (A + 1)."""
+        return PolicyInputSchema(self._policy_input_layout(),
+                                 self_columns=(tuple(input_column(h) for h in self.agent_observation_bounds), ),
+                                 task_columns=tuple(input_column(h, none) for h, none in
+                                                    zip(self.passenger_observation_bounds, self._NONE_TASK_COLUMNS)))
+
+    def _inputs_entry(self):
+        return self._lib.frz_rideshare_policy_inputs
 
     # ------------------------------------------------------------------------------------------ logging tap
 

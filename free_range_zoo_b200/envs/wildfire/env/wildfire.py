@@ -19,7 +19,8 @@ from free_range_zoo_b200.utils.containers import (LazyDict, ObservationDict, jag
                                                   jagged_indices_from_mask)
 from free_range_zoo_b200.utils.conversions import batched_aec_to_batched_parallel
 from free_range_zoo_b200.utils import compact
-from free_range_zoo_b200.utils.env import AutoresetRows, BatchedAECEnv
+from free_range_zoo_b200.utils.env import (AutoresetRows, BatchedAECEnv, InputKind, PolicyInputLayout,
+                                           PolicyInputSchema, input_column)
 from free_range_zoo_b200.utils.spaces import BatchedActionSpace, Space
 
 
@@ -369,6 +370,23 @@ class raw_env(BatchedAECEnv):
 
     def _policy_entry(self):
         return self._lib.frz_wildfire_policy_actions
+
+    def _policy_input_layout(self) -> PolicyInputLayout:
+        """Self (y, x, power, suppressant), of the others y, x and the observed power / suppressant; task rows
+        (y, x, fire type, intensity), one view."""
+        observed = (0, 1) + ((2, ) if self.observe_other_power else ()) + ((3, ) if self.observe_other_suppressant else ())
+        p = self._params
+        return PolicyInputLayout(kinds=(InputKind(int(p.num_agents), 4, observed), ), task_rows=int(p.height) * int(p.width),
+                                 views=1, task_columns=(False, ) * 4)
+
+    def _policy_input_schema(self) -> PolicyInputSchema:
+        """``1 / high`` of ``agent_observation_bounds`` and ``fire_observation_bounds``."""
+        return PolicyInputSchema(self._policy_input_layout(),
+                                 self_columns=(tuple(input_column(h) for h in self.agent_observation_bounds), ),
+                                 task_columns=tuple(input_column(h) for h in self.fire_observation_bounds))
+
+    def _inputs_entry(self):
+        return self._lib.frz_wildfire_policy_inputs
 
     # ------------------------------------------------------------------------------------------ logging tap
 

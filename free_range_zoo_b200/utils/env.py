@@ -51,6 +51,41 @@ class AutoresetRows(NamedTuple):
     final: Tuple[str, ...]
 
 
+class InputKind(NamedTuple):
+    """Agents of one kind in the policy inputs: ``count`` agents (consecutive in the action table) whose self table
+    has ``columns`` columns, of which ``observed`` appear for every other agent of the kind in its ``others`` view."""
+    count: int
+    columns: int
+    observed: Tuple[int, ...]
+
+    @property
+    def width(self) -> int:
+        return self.columns + (self.count - 1) * len(self.observed)
+
+
+class PolicyInputLayout(NamedTuple):
+    """The structure of the policy inputs (include/frz_inputs.h)."""
+    kinds: Tuple[InputKind, ...]  # one, or cybersecurity's attackers and defenders
+    task_rows: int  # T
+    views: int  # V
+    task_columns: Tuple[bool, ...]  # one per task_obs column: True for a "none" column whose FRZ_PAD means nobody
+    flags: int = 0  # _lib.INPUTS_*
+
+
+class PolicyInputSchema(NamedTuple):
+    """A layout and the ``(scale, offset)`` of every source column (self columns per kind, then task columns)."""
+    layout: PolicyInputLayout
+    self_columns: Tuple[Tuple[Tuple[float, int], ...], ...]
+    task_columns: Tuple[Tuple[float, int], ...]
+
+
+def input_column(high, none: bool = False) -> Tuple[float, int]:
+    """``(scale, offset)`` of a column bounded by ``high``: ``(1 / high, 0)``, or ``(1 / (high + 1), 1)`` for a "none"
+    column (its "none" value -1 then maps to 0); scale 1 where the bound is missing or not positive."""
+    high = None if high is None else float(high) + (1.0 if none else 0.0)
+    return (1.0 if high is None or not high > 0 else 1.0 / high), (1 if none else 0)
+
+
 class _DeviceBound:
     """libfrz entry points bound to one CUDA device: every call of the C ABI works on the CURRENT device
     (include/frz.h), so calls made while another device is current switch to the environment's device for their
@@ -1011,3 +1046,113 @@ class BatchedAECEnv(ABC):
             buffers['slots'].copy_(slots, non_blocking=True)
         self._policy_launch(_lib.POLICY_DECODE)
         return self._actions
+
+    # ------------------------------------------------------------------------------------------ policy inputs
+
+    def _policy_input_layout(self) -> PolicyInputLayout:
+        """The structure of the policy inputs (include/frz_inputs.h), from ``_params`` and the observe flags only (no
+        device, no configuration).  Domain hook."""
+        raise NotImplementedError
+
+    def _policy_input_schema(self) -> PolicyInputSchema:
+        """The layout and every column's ``(scale, offset)``, from the bounds of ``observation_space``.  Domain hook."""
+        raise NotImplementedError
+
+    def _inputs_entry(self):
+        """The domain's ``frz_<domain>_policy_inputs`` entry point."""
+        raise NotImplementedError
+
+    @property
+    def policy_input_shapes(self) -> Dict[str, Tuple[int, ...]]:
+        """``{'agent': (A, Fa), 'tasks': (V, T, Ft)}``: the per-environment shapes of ``policy_inputs``.  Row t < T of
+        a view's task block is padded task row t, which action slot t acts on (``action_slots``): wildfire env-local
+        task t, rideshare table row t, cybersecurity node t."""
+        layout = self._policy_input_layout()
+        A = sum(kind.count for kind in layout.kinds)
+        Fa = max(kind.width for kind in layout.kinds if kind.count > 0)
+        return {'agent': (A, Fa), 'tasks': (layout.views, layout.task_rows, len(layout.task_columns) + 1)}
+
+    def _policy_inputs_block(self) -> _lib.PolicyInputs:
+        """The launch block with the schema's column tables (built once; the call fills in outputs and type)."""
+        block = self.__dict__.get('_inputs_block')
+        if block is None:
+            schema = self._policy_input_schema()
+            layout = schema.layout
+            block = _lib.PolicyInputs()
+            shapes = self.policy_input_shapes
+            block.agent_width = shapes['agent'][1]
+            block.views, block.task_rows, block.task_width = shapes['tasks']
+            block.flags = layout.flags
+            for index, (kind, columns) in enumerate(zip(layout.kinds, schema.self_columns)):
+                target = block.self_columns[index]
+                target.columns = kind.columns
+                target.observed = sum(1 << c for c in kind.observed)
+                for c, (scale, offset) in enumerate(columns):
+                    target.scale[c], target.offset[c] = scale, offset
+            target = block.task_columns
+            target.columns = len(layout.task_columns)
+            target.pad_is_none = sum(1 << c for c, none in enumerate(layout.task_columns) if none)
+            for c, (scale, offset) in enumerate(schema.task_columns):
+                target.scale[c], target.offset[c] = scale, offset
+            self._inputs_block = block
+        return block
+
+    def _inputs_io(self, final: bool):
+        """The domain's buffer struct, with the observation arrays of ``final_observations`` when ``final``."""
+        if not final:
+            return self._io
+        if not self.keep_final_observations:
+            raise RuntimeError('final_observations are kept by the autoreset: construct the environment with '
+                               'autoreset=True, keep_final_observations=True')
+        io = type(self._io).from_buffer_copy(self._io)
+        for name, tensor in self._final_buffers.items():
+            setattr(io, name, tensor.data_ptr())
+        return io
+
+    def policy_inputs(self, dtype: torch.dtype = torch.float32, final: bool = False,
+                      out: Optional[Tuple[torch.Tensor, torch.Tensor]] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+        """The observations of every environment and agent as fixed-width policy inputs (include/frz_inputs.h), in one
+        launch with no host read (capturable in a CUDA graph).  Returns ``(agent, tasks)`` of ``dtype`` (f32 or bf16):
+
+        - ``agent`` [B, A, Fa]: the agent's ``self`` columns, then the observed columns of each agent of its ``others``
+          view, in the view's order (cybersecurity: the shorter kind zero-padded);
+        - ``tasks`` [B, V, T, Ft]: row t is padded task row t, i.e. action slot t.  Column 0 is 1 iff the row is a live
+          task the view may see, then the row's columns; other rows are all zeros.  V = 1 when every agent sees the same
+          tasks (wildfire, rideshare), V = A when views differ (cybersecurity: an unmonitored defender under partial
+          observability sees none).
+
+        Every column is ``float(v + offset) * scale`` in f32 (bf16: rounded once, to nearest even), with scale
+        ``1 / high`` of the column's bound in ``observation_space`` (1 where a bound is missing or not positive) and
+        offset 0; "none" columns (rideshare accepted_by / riding_by, the cybersecurity defender location) use offset 1
+        and scale ``1 / (high + 1)``, so that "none" is exactly 0.  No clamping.
+
+        ``final=True`` encodes ``final_observations`` (``keep_final_observations=True`` only).  The result buffers
+        belong to the environment, one pair per ``(dtype, final)``, allocated by the first call and overwritten by the
+        next; ``out=(agent, tasks)`` writes into contiguous caller tensors of the right shape, dtype and device instead
+        (e.g. ``storage[t]`` of a ``[T_rollout, B, ...]`` rollout buffer)."""
+        if dtype not in (torch.float32, torch.bfloat16):
+            raise ValueError(f'dtype must be torch.float32 or torch.bfloat16, not {dtype}')
+        io = self._inputs_io(final)
+        shapes = self.policy_input_shapes
+        B = self.parallel_envs
+        wanted = ((B, ) + shapes['agent'], (B, ) + shapes['tasks'])
+        if out is None:
+            buffers = self.__dict__.setdefault('_inputs', {})
+            out = buffers.get((dtype, final))
+            if out is None:
+                out = buffers[(dtype, final)] = tuple(torch.zeros(shape, dtype=dtype, device=self.device)
+                                                      for shape in wanted)
+        else:
+            if not isinstance(out, (tuple, list)) or len(out) != 2:
+                raise ValueError('out must be a pair (agent, tasks)')
+            for name, tensor, shape in zip(('agent', 'tasks'), out, wanted):
+                if not isinstance(tensor, torch.Tensor) or tuple(tensor.shape) != shape or tensor.dtype != dtype \
+                        or tensor.device != self.device or not tensor.is_contiguous():
+                    raise ValueError(f'out {name} must be a contiguous {dtype} tensor of shape {shape} on {self.device}')
+            out = tuple(out)
+        block = _lib.PolicyInputs.from_buffer_copy(self._policy_inputs_block())
+        block.agent, block.tasks = out[0].data_ptr(), out[1].data_ptr()
+        block.output_type = _lib.INPUTS_BF16 if dtype == torch.bfloat16 else _lib.INPUTS_F32
+        _lib.check(self._inputs_entry()(ctypes.byref(self._params), ctypes.byref(io), B, ctypes.byref(block),
+                                        self._stream()), 'policy_inputs')
+        return out
