@@ -209,6 +209,18 @@ class PolicyInputs(C.Structure):
 INPUTS_F32, INPUTS_BF16 = 0, 1
 INPUTS_PARTIALLY_OBSERVABLE = 0x1
 
+
+class Advantages(C.Structure):
+    """FrzAdvantages (include/frz_returns.h): sizes, discounts, inputs and outputs of one GAE launch.  (``lambda`` is a
+    Python keyword: set it with ``setattr``.)"""
+    _fields_ = [('T', C.c_int32), ('B', C.c_int32), ('A', C.c_int32), ('value_type', C.c_int32), ('gamma', C.c_float),
+                ('lambda', C.c_float), ('rewards', C.c_void_p), ('values', C.c_void_p), ('next_values', C.c_void_p),
+                ('final_values', C.c_void_p), ('terminated', C.c_void_p), ('truncated', C.c_void_p),
+                ('advantages', C.c_void_p), ('returns', C.c_void_p)]
+
+
+VALUES_F32, VALUES_BF16 = 0, 1
+
 OBS_DENSE, OBS_ROWS, OBS_MASK_BITS = 0, 1, 2
 OBS_I32, OBS_I16, OBS_I8, OBS_U8, OBS_F32 = 0, 1, 2, 3, 4
 HOST_ACTIONS_I32, HOST_ACTIONS_I16, HOST_ACTIONS_I8 = 0, 1, 2
@@ -267,6 +279,7 @@ def library() -> C.CDLL:
                                   ('frz_rideshare_policy_inputs', RideshareParams, RideshareBuffers)):
         getattr(lib, name).argtypes = [C.POINTER(params), C.POINTER(buffers), C.c_int32, C.POINTER(PolicyInputs),
                                        C.c_void_p]
+    lib.frz_advantages.argtypes = [C.POINTER(Advantages), C.c_void_p]
     if lib.frz_version() != ABI_VERSION:
         raise RuntimeError(f'libfrz.so ABI version {lib.frz_version()} != {ABI_VERSION}; rebuild the library')
     lib.frz_control_restore.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p]

@@ -336,6 +336,14 @@ class BatchedAECEnv(ABC):
             return {agent: self._zero_rewards for agent in self.agents}
         return self._reward_views
 
+    @property
+    def reward_table(self) -> torch.Tensor:
+        """f32 [B, A] on the device: the rewards of the last environment step, agents in the order of ``possible_agents``.
+        It is the buffer ``rewards[agent]`` views column by column and keeps its address on every step, so a rollout
+        stores a step with one ``storage[t].copy_(env.reward_table)`` (capturable).  The next step overwrites it; unlike
+        ``rewards`` it is not zeroed in the middle of an AEC round, and ``detach_outputs`` does not copy it."""
+        return self._rewards
+
     # ------------------------------------------------------------------------------------------ allocation
 
     def _allocate_runtime(self, num_agents: int) -> None:
