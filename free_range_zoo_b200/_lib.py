@@ -188,6 +188,7 @@ class PolicyActions(C.Structure):
 
 
 POLICY_SAMPLE, POLICY_DECODE, POLICY_LEGAL = 0, 1, 2
+POLICY_PACKED_LEGAL = 0x100
 LOGITS_F32, LOGITS_BF16 = 0, 1
 
 INPUTS_MAX_COLUMNS = 8
@@ -220,6 +221,19 @@ class Advantages(C.Structure):
 
 
 VALUES_F32, VALUES_BF16 = 0, 1
+
+
+class SlotLogProb(C.Structure):
+    """FrzSlotLogProb (include/frz_logprob.h): rows, logits, mask, chosen slots, outputs and incoming gradients of one
+    masked log-probability / entropy launch (forward or backward)."""
+    _fields_ = [('rows', C.c_int64), ('slots', C.c_int32), ('row_stride', C.c_int32), ('logits_type', C.c_int32),
+                ('legal_type', C.c_int32), ('logits', C.c_void_p), ('legal', C.c_void_p), ('slot', C.c_void_p),
+                ('log_prob', C.c_void_p), ('entropy', C.c_void_p), ('grad_log_prob', C.c_void_p),
+                ('grad_entropy', C.c_void_p), ('grad_logits', C.c_void_p)]
+
+
+MASK_BYTES, MASK_BITS = 0, 1
+SLOT_LOG_PROB_MAX_SLOTS = 288
 
 OBS_DENSE, OBS_ROWS, OBS_MASK_BITS = 0, 1, 2
 OBS_I32, OBS_I16, OBS_I8, OBS_U8, OBS_F32 = 0, 1, 2, 3, 4
@@ -280,6 +294,8 @@ def library() -> C.CDLL:
         getattr(lib, name).argtypes = [C.POINTER(params), C.POINTER(buffers), C.c_int32, C.POINTER(PolicyInputs),
                                        C.c_void_p]
     lib.frz_advantages.argtypes = [C.POINTER(Advantages), C.c_void_p]
+    for name in ('frz_slot_log_prob', 'frz_slot_log_prob_backward'):
+        getattr(lib, name).argtypes = [C.POINTER(SlotLogProb), C.c_void_p]
     if lib.frz_version() != ABI_VERSION:
         raise RuntimeError(f'libfrz.so ABI version {lib.frz_version()} != {ABI_VERSION}; rebuild the library')
     lib.frz_control_restore.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p]

@@ -1,9 +1,10 @@
 // Policy actions from logits over the fixed-width slot layout (frz_<domain>_policy_actions, include/frz_policy.h).
 //
-// One launch, a group of G lanes per (environment, agent) row; slot t of a row belongs to lane t % G of its group, in
-// round t / G, so every round's loads of a group are consecutive elements (coalesced, no alignment needed, any row
-// stride).  G is chosen from C: one thread per row for C <= 16 (cybersecurity, small wildfire grids), else the
-// smallest group that leaves at most 4 slots per lane, up to a warp (9 slots per lane for the largest grids).
+// One launch, a group of G lanes per (environment, agent) row, the row mapping of frz_slots.cuh: slot t of a row belongs
+// to lane t % G of its group, in round t / G, so every round's loads of a group are consecutive elements (coalesced, no
+// alignment needed, any row stride).  G is chosen from C: one thread per row for C <= 16 (cybersecurity, small wildfire
+// grids), else the smallest group that leaves at most 4 slots per lane, up to a warp (9 slots per lane for the largest
+// grids).
 //   pass 1  legality of every slot from the domain's own buffers (the Rule below), in registers; SAMPLE loads the
 //           legal slots' logits, checks them and reduces their max m over the group
 //   pass 2  SAMPLE: running sums of exp(l - m) in slot order, round by round (group inclusive scan + the carry of the
@@ -11,7 +12,8 @@
 //   pass 3  the target slot, uniform over the group: SAMPLE the first legal slot whose running sum exceeds u * S (the
 //           last legal slot if none does), DECODE the caller's slot; the noop on a fault
 //   pass 4  the lane owning the target writes the action (k = the slot's rank among the legal slots, its id), the slot
-//           and the log-probability; every lane writes its legality bytes when asked to
+//           and the log-probability; every lane writes its legality bytes when asked to (with
+//           FRZ_POLICY_PACKED_LEGAL, lane 0 of the group writes the row's words, built from the rounds' ballots)
 // Equal logits: every exp term is exactly 1 and S is the exact count n + 1, so u * S is the single multiply of the
 // uniform sampler (u01(r.x) * float(n + 1)) and the first running sum above it is at choice int(u * S): the choice is
 // exactly frz_<domain>_sample_actions'.
@@ -19,6 +21,7 @@
 
 #include "frz_common.cuh"
 #include "frz_policy.h"
+#include "frz_slots.cuh"
 
 namespace frz {
 namespace {
@@ -115,15 +118,10 @@ struct Launch {
 __device__ __forceinline__ float logit(const float* p) { return *p; }
 __device__ __forceinline__ float logit(const __nv_bfloat16* p) { return __bfloat162float(*p); }
 
-// the G-lane group's bits of a warp-wide predicate
-template <int G>
-__device__ __forceinline__ uint32_t group_ballot(bool predicate, int base) {
-  const uint32_t all = __ballot_sync(kFullMask, predicate);
-  return G == 32 ? all : (all >> base) & ((1u << G) - 1u);
-}
-
-template <class Rule, int G, int PER, class T>
-__global__ void __launch_bounds__(kPolicyThreads) policy_kernel(const Rule rule, const Launch L) {
+// PACKED: `legal` receives the packed words of include/frz_policy.h instead of bytes.  (Its minimum of one CTA per SM
+// lets ptxas use the registers it needs instead of spilling a few bytes; 0 leaves the byte instantiations as they were.)
+template <class Rule, int G, int PER, class T, bool PACKED>
+__global__ void __launch_bounds__(kPolicyThreads, PACKED ? 1 : 0) policy_kernel(const Rule rule, const Launch L) {
   const FrzPolicyActions& P = L.policy;
   const int lane = threadIdx.x & 31, glane = lane & (G - 1), base = lane - glane;
   const int C = rule.C, A = rule.A;
@@ -157,7 +155,26 @@ __global__ void __launch_bounds__(kPolicyThreads) policy_kernel(const Rule rule,
         bad |= l[j] != l[j] || l[j] == INFINITY;
         m = fmaxf(m, l[j]);
       }
-      if (P.legal != nullptr && active && t < C) P.legal[size_t(row) * C + t] = ok;
+      if (!PACKED && P.legal != nullptr && active && t < C) P.legal[size_t(row) * C + t] = ok;
+    }
+    if (PACKED && P.legal != nullptr) {
+      // round j's group ballot holds slots j * G .. j * G + G - 1, at shift (j * G) % 32 of word (j * G) / 32; a word
+      // is stored as soon as its last round is in
+      uint32_t* words = reinterpret_cast<uint32_t*>(P.legal) + size_t(row) * size_t((C + 31) / 32);
+      const bool store = active && glane == 0;
+      if (G == 1) {
+        if (store) words[0] = legal_bits;
+      } else {
+        uint32_t word = 0u;
+#pragma unroll
+        for (int j = 0; j < PER; ++j) {
+          word |= group_ballot<G>(legal_bits >> j & 1u, base) << (j * G % 32);
+          if ((j + 1) * G % 32 == 0 || j == PER - 1) {
+            if (store && j * G / 32 * 32 < C) words[j * G / 32] = word;
+            word = 0u;
+          }
+        }
+      }
     }
     if (P.mode == FRZ_POLICY_LEGAL) continue;
 
@@ -170,16 +187,7 @@ __global__ void __launch_bounds__(kPolicyThreads) policy_kernel(const Rule rule,
       // pass 2: running sums in slot order
       float running[PER];
 #pragma unroll
-      for (int j = 0; j < PER; ++j) {
-        float x = (legal_bits >> j & 1u) ? (l[j] == m ? 1.f : expf(l[j] - m)) : 0.f;
-#pragma unroll
-        for (int o = 1; o < G; o <<= 1) {
-          const float y = __shfl_up_sync(kFullMask, x, o, G);
-          if (glane >= o) x += y;
-        }
-        running[j] = S + x;
-        S += __shfl_sync(kFullMask, x, G - 1, G);
-      }
+      for (int j = 0; j < PER; ++j) running[j] = running_sum<G>(slot_term(legal_bits >> j & 1u, l[j], m), glane, S);
       // pass 3: the first legal slot whose running sum exceeds u * S, else the last legal slot
       const uint64_t genv = uint64_t(L.env_offset + env);
       const uint4 bits = philox(uint32_t(genv), uint32_t(step), 0xC0000000u | uint32_t(agent),
@@ -230,27 +238,29 @@ __global__ void __launch_bounds__(kPolicyThreads) policy_kernel(const Rule rule,
 
 // ---------------------------------------------------------------------------------------------- launch
 
-template <class Rule, int G, int PER>
-int launch_typed(const Rule& rule, const Launch& launch, cudaStream_t stream) {
+template <class Rule, int G, int PER, bool PACKED>
+void launch_typed(const Rule& rule, const Launch& launch, cudaStream_t stream) {
   const int64_t threads = int64_t(launch.rows) * G;
   const int work_ctas = int((threads + kPolicyThreads - 1) / kPolicyThreads);
   const int grid = persistent_grid(work_ctas, 2048 / kPolicyThreads);
   if (launch.policy.mode == FRZ_POLICY_SAMPLE && launch.policy.logits_type == FRZ_LOGITS_BF16)
-    policy_kernel<Rule, G, PER, __nv_bfloat16><<<grid, kPolicyThreads, 0, stream>>>(rule, launch);
+    policy_kernel<Rule, G, PER, __nv_bfloat16, PACKED><<<grid, kPolicyThreads, 0, stream>>>(rule, launch);
   else
-    policy_kernel<Rule, G, PER, float><<<grid, kPolicyThreads, 0, stream>>>(rule, launch);
-  return check_launch("policy_kernel");
+    policy_kernel<Rule, G, PER, float, PACKED><<<grid, kPolicyThreads, 0, stream>>>(rule, launch);
 }
 
-// lanes per row and slots per lane from C (<= FRZ_MAX_CELLS + 1)
+// lanes per row and slots per lane from C (<= FRZ_MAX_CELLS + 1), legality bytes or packed words
 template <class Rule>
-int launch(const Rule& rule, const Launch& launch, cudaStream_t stream) {
-  const int C = rule.C;
-  if (C <= 16) return launch_typed<Rule, 1, 16>(rule, launch, stream);
-  if (C <= 32) return launch_typed<Rule, 8, 4>(rule, launch, stream);
-  if (C <= 64) return launch_typed<Rule, 16, 4>(rule, launch, stream);
-  if (C <= 128) return launch_typed<Rule, 32, 4>(rule, launch, stream);
-  return launch_typed<Rule, 32, 9>(rule, launch, stream);
+int launch(const Rule& rule, const Launch& launch, bool packed, cudaStream_t stream) {
+  with_row_mapping(rule.C, [&](auto map) {
+    using M = decltype(map);
+    if (packed)
+      launch_typed<Rule, M::G, M::PER, true>(rule, launch, stream);
+    else
+      launch_typed<Rule, M::G, M::PER, false>(rule, launch, stream);
+    return 0;
+  });
+  return check_launch("policy_kernel");
 }
 
 // argument checks shared by the three domains; fills `launch`
@@ -260,19 +270,18 @@ int check_policy(const FrzPolicyActions* policy, int32_t* actions, FrzControl* c
     set_error("%s: NULL params / buffers / policy block", what);
     return FRZ_ERR_NULL;
   }
-  if (policy->mode != FRZ_POLICY_SAMPLE && policy->mode != FRZ_POLICY_DECODE && policy->mode != FRZ_POLICY_LEGAL) {
+  const int mode = policy->mode & ~int32_t(FRZ_POLICY_PACKED_LEGAL);
+  if (mode != FRZ_POLICY_SAMPLE && mode != FRZ_POLICY_DECODE && mode != FRZ_POLICY_LEGAL) {
     set_error("%s: unknown mode %d", what, policy->mode);
     return FRZ_ERR_UNSUPPORTED;
   }
-  if (policy->mode == FRZ_POLICY_SAMPLE && policy->logits_type != FRZ_LOGITS_F32 &&
-      policy->logits_type != FRZ_LOGITS_BF16) {
+  if (mode == FRZ_POLICY_SAMPLE && policy->logits_type != FRZ_LOGITS_F32 && policy->logits_type != FRZ_LOGITS_BF16) {
     set_error("%s: unknown logits type %d", what, policy->logits_type);
     return FRZ_ERR_UNSUPPORTED;
   }
-  if ((policy->mode == FRZ_POLICY_SAMPLE && (policy->logits == nullptr || policy->slot == nullptr)) ||
-      (policy->mode == FRZ_POLICY_DECODE && policy->slot == nullptr) ||
-      (policy->mode != FRZ_POLICY_LEGAL && actions == nullptr) ||
-      (policy->mode == FRZ_POLICY_LEGAL && policy->legal == nullptr)) {
+  if ((mode == FRZ_POLICY_SAMPLE && (policy->logits == nullptr || policy->slot == nullptr)) ||
+      (mode == FRZ_POLICY_DECODE && policy->slot == nullptr) || (mode != FRZ_POLICY_LEGAL && actions == nullptr) ||
+      (mode == FRZ_POLICY_LEGAL && policy->legal == nullptr)) {
     set_error("%s: a pointer the mode needs is NULL", what);
     return FRZ_ERR_NULL;
   }
@@ -284,11 +293,16 @@ int check_policy(const FrzPolicyActions* policy, int32_t* actions, FrzControl* c
     set_error("%s: slots=%d, but this configuration has %d", what, policy->slots, C);
     return FRZ_ERR_SHAPE;
   }
-  if (policy->mode == FRZ_POLICY_SAMPLE && policy->row_stride < C) {
+  if (mode == FRZ_POLICY_SAMPLE && policy->row_stride < C) {
     set_error("%s: row_stride=%d < slots=%d", what, policy->row_stride, C);
     return FRZ_ERR_SHAPE;
   }
+  if ((policy->mode & FRZ_POLICY_PACKED_LEGAL) != 0 && reinterpret_cast<uintptr_t>(policy->legal) % 4 != 0) {
+    set_error("%s: packed legal mask is not 4-byte aligned", what);
+    return FRZ_ERR_SHAPE;
+  }
   launch->policy = *policy;
+  launch->policy.mode = mode;
   launch->actions = actions;
   launch->control = control;
   launch->rows = B * A;
@@ -330,7 +344,7 @@ int frz_wildfire_policy_actions(const FrzWildfireParams* params, const FrzWildfi
   launch.env_offset = params->env_offset;
   const WildfireRule rule{io->action_mask, io->env_task_count, params->num_agents, cells + 1, cells, io->mask_stride,
                           show_bad};
-  return frz::launch(rule, launch, static_cast<cudaStream_t>(stream));
+  return frz::launch(rule, launch, (policy->mode & FRZ_POLICY_PACKED_LEGAL) != 0, static_cast<cudaStream_t>(stream));
 }
 
 int frz_rideshare_policy_actions(const FrzRideshareParams* params, const FrzRideshareBuffers* io,
@@ -355,7 +369,7 @@ int frz_rideshare_policy_actions(const FrzRideshareParams* params, const FrzRide
   }
   launch.env_offset = params->env_offset;
   const RideshareRule rule{io->task_mask, io->task_obs, params->num_agents, params->capacity + 1, params->capacity, 0};
-  return frz::launch(rule, launch, static_cast<cudaStream_t>(stream));
+  return frz::launch(rule, launch, (policy->mode & FRZ_POLICY_PACKED_LEGAL) != 0, static_cast<cudaStream_t>(stream));
 }
 
 int frz_cyber_policy_actions(const FrzCyberParams* params, const FrzCyberBuffers* io, int32_t parallel_envs,
@@ -386,7 +400,7 @@ int frz_cyber_policy_actions(const FrzCyberParams* params, const FrzCyberBuffers
   launch.env_offset = params->env_offset;
   const CyberRule rule{io->env_task_count, io->agent_task_count, io->location, A, params->num_nodes + 3,
                        params->num_nodes, params->num_attackers, show_bad};
-  return frz::launch(rule, launch, static_cast<cudaStream_t>(stream));
+  return frz::launch(rule, launch, (policy->mode & FRZ_POLICY_PACKED_LEGAL) != 0, static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

@@ -983,6 +983,20 @@ class BatchedAECEnv(ABC):
                                           legal=torch.zeros((B, A, self.action_slots), dtype=torch.bool, device=dev))
         return buffers
 
+    def _legal_kind(self, tensor: torch.Tensor, what: str) -> bool:
+        """Check a legal-mask output: bool / uint8 [B, A, C], or int32 [B, A, W] (W = ceil(C / 32)) for the packed mask
+        (include/frz_policy.h), contiguous.  Returns whether it is packed."""
+        B, A, C = self.parallel_envs, len(self.possible_agents), self.action_slots
+        packed = isinstance(tensor, torch.Tensor) and tensor.dtype == torch.int32
+        if not packed:
+            self._check_policy_tensor(tensor, what, (torch.bool, torch.uint8))
+        elif tensor.device != self.device or tuple(tensor.shape) != (B, A, (C + 31) // 32):
+            raise ValueError(f'{what} (packed) must be an int32 tensor of shape {(B, A, (C + 31) // 32)} on '
+                             f'{self.device} (W = ceil({C} / 32) words per row)')
+        if not tensor.is_contiguous():
+            raise ValueError(f'{what} must be contiguous')
+        return packed
+
     def _check_policy_tensor(self, tensor: torch.Tensor, what: str, dtypes, slots: bool = True) -> None:
         B, A = self.parallel_envs, len(self.possible_agents)
         shape = (B, A, self.action_slots) if slots else (B, A)
@@ -995,6 +1009,8 @@ class BatchedAECEnv(ABC):
                        sampler_seed: int = 0) -> None:
         buffers = self._policy_buffers()
         block = _lib.PolicyActions()
+        if legal is not None and legal.dtype == torch.int32:
+            mode |= _lib.POLICY_PACKED_LEGAL
         block.mode, block.slots = mode, self.action_slots
         block.slot, block.log_prob = buffers['slots'].data_ptr(), buffers['log_prob'].data_ptr()
         block.legal = _lib.pointer(legal)
@@ -1005,15 +1021,21 @@ class BatchedAECEnv(ABC):
         _lib.check(self._policy_entry()(ctypes.byref(self._params), ctypes.byref(self._io), self.parallel_envs,
                                         ctypes.byref(block), self._stream()), 'policy_actions')
 
-    def legal_actions(self, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def legal_actions(self, out: Optional[torch.Tensor] = None, packed: bool = False) -> torch.Tensor:
         """bool [B, A, C] on the device: slot t of (environment, agent) is legal (``action_slots``).  Written into
-        ``out`` (bool or uint8, contiguous) when given, else into an env-owned buffer the next call overwrites."""
+        ``out`` (bool or uint8, contiguous) when given, else into an env-owned buffer the next call overwrites.
+
+        ``packed=True`` returns the mask bit-packed instead, int32 [B, A, W] with W = ceil(C / 32): bit t % 32 of word
+        t / 32 is slot t, bits at or beyond C are 0 (``utils.policy.unpack_legal`` unpacks it).  An int32 ``out`` of
+        that shape receives the packed mask too."""
         if out is None:
-            out = self._policy_buffers()['legal']
+            buffers = self._policy_buffers()
+            if packed and 'legal_packed' not in buffers:
+                B, A, C = self.parallel_envs, len(self.possible_agents), self.action_slots
+                buffers['legal_packed'] = torch.zeros((B, A, (C + 31) // 32), dtype=torch.int32, device=self.device)
+            out = buffers['legal_packed' if packed else 'legal']
         else:
-            self._check_policy_tensor(out, 'out', (torch.bool, torch.uint8))
-            if not out.is_contiguous():
-                raise ValueError('out must be contiguous')
+            self._legal_kind(out, 'out')
         self._policy_launch(_lib.POLICY_LEGAL, legal=out)
         return out
 
@@ -1024,8 +1046,10 @@ class BatchedAECEnv(ABC):
         ``step_all(None)`` / the Parallel ``step``.  One launch, no host read: capturable in a CUDA graph.
 
         Returns ``(slots, log_prob)``: int32 [B, A] chosen slots and f32 [B, A] their log-probability under the masked
-        softmax, env-owned buffers overwritten by the next call.  ``legal_out`` (bool / uint8 [B, A, C], contiguous)
-        receives the legal mask in the same launch, e.g. for a learner that recomputes log-probabilities with gradients.
+        softmax, env-owned buffers overwritten by the next call.  ``legal_out`` (bool / uint8 [B, A, C], or int32
+        [B, A, ceil(C / 32)] for the packed mask of ``legal_actions(packed=True)``; contiguous) receives the legal mask
+        in the same launch, e.g. for a learner that recomputes log-probabilities with gradients
+        (``utils.policy.slot_log_prob``).
         The random draw of (environment, agent) is the one ``sample_actions(sampler_seed)`` makes, so equal logits
         stage exactly what ``sample_actions`` stages.  NaN / +inf in a legal slot, or -inf in all of them, records a
         fault (``check_errors``) and stages the noop."""
@@ -1034,9 +1058,7 @@ class BatchedAECEnv(ABC):
             raise ValueError('logits rows must be evenly spaced with unit stride along the slots '
                              '(a contiguous tensor, or a [..., :C] view of one)')
         if legal_out is not None:
-            self._check_policy_tensor(legal_out, 'legal_out', (torch.bool, torch.uint8))
-            if not legal_out.is_contiguous():
-                raise ValueError('legal_out must be contiguous')
+            self._legal_kind(legal_out, 'legal_out')
         self._policy_launch(_lib.POLICY_SAMPLE, logits=logits, legal=legal_out, sampler_seed=sampler_seed)
         buffers = self._policy_buffers()
         return buffers['slots'], buffers['log_prob']

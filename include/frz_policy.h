@@ -33,6 +33,11 @@
  *   FRZ_POLICY_LEGAL   legal[row, t] <- 1 iff slot t is legal (nothing else is written).
  * legal (optional in the first two modes) receives the same mask.  bf16 logits are widened to f32 on load.
  *
+ * FRZ_POLICY_PACKED_LEGAL may be OR-ed into any mode: legal then receives the mask bit-packed, as uint32 [B, A, W] with
+ * W = ceil(C / 32) words per row.  Bit t % 32 of word t / 32 is slot t; bits at or beyond C are 0.  The pointer must be
+ * 4-byte aligned (FRZ_ERR_SHAPE otherwise).  This is the packed layout that frz_logprob.h reads; a rollout that stores
+ * it keeps 4 * W bytes per row instead of C (16 instead of 101 at wildfire C4).
+ *
  * Faults (bits of FrzControl.error_word; the row is decoded as the noop): FRZ_FAULT_BAD_LOGITS when a legal slot's logit
  * is NaN or +inf or every legal logit is -inf (its log_prob is NaN), FRZ_FAULT_ILLEGAL_SLOT when a DECODE slot is out of
  * [0, C) or illegal.  Logits of illegal slots are never read.
@@ -54,19 +59,20 @@ extern "C" {
 #define FRZ_POLICY_SAMPLE 0
 #define FRZ_POLICY_DECODE 1
 #define FRZ_POLICY_LEGAL 2
+#define FRZ_POLICY_PACKED_LEGAL 0x100 /* flag: legal is the packed uint32 [B, A, ceil(C / 32)] mask */
 
 #define FRZ_LOGITS_F32 0
 #define FRZ_LOGITS_BF16 1
 
 typedef struct {
-  int32_t mode;          /* FRZ_POLICY_* */
+  int32_t mode;          /* FRZ_POLICY_*, optionally | FRZ_POLICY_PACKED_LEGAL */
   int32_t logits_type;   /* FRZ_LOGITS_* */
   const void* logits;    /* device [B, A, row_stride], the first `slots` of each row used (SAMPLE) */
   int32_t slots;         /* C of the configuration (checked) */
   int32_t row_stride;    /* elements between consecutive rows of logits, >= slots */
   int32_t* slot;         /* device int32 [B, A]: out (SAMPLE), in (DECODE) */
   float* log_prob;       /* device f32 [B, A] out (SAMPLE), or NULL */
-  uint8_t* legal;        /* device u8 [B, A, slots] out, or NULL (required for LEGAL) */
+  uint8_t* legal;        /* device u8 [B, A, slots] (packed: uint32 [B, A, W]) out, or NULL (required for LEGAL) */
   uint64_t sampler_seed; /* Philox key of SAMPLE, as for frz_<domain>_sample_actions */
 } FrzPolicyActions;
 
